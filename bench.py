@@ -13,9 +13,13 @@ independent batch; the only collective is the NCCL all-reduce of the pool-parame
 stream so that it overlaps the next step's forward.
 
 Timing: a measurement is EXACTLY --steps steps between two CUDA events, bracketed by a barrier and a
-device synchronisation on both sides, max over ranks.  That measurement is repeated (`rounds`, sized
-so that the timed regions add up to >= 2.5 s) and the MEDIAN round is reported; every round, the mean
-and per-rank step statistics are in `consistency`.
+device synchronisation on both sides, max over ranks.  By default it is taken once, so the timed steps
+are exactly --steps; --rounds R repeats it R times (0: as many rounds as add up to >= 2.5 s) and the
+MEDIAN round is reported; every round, the mean and per-rank step statistics are in `consistency`.
+
+--dump-outputs DIR writes what the timed path returned in its last timed step (out [N,C], gx [V,C],
+gcompat [V,G], ggate [2,G]) as DIR/<name>.npy in float32, each array capped at 16 MB by a fixed seeded
+sample of its rows, so that two builds run with the same arguments can be compared output for output.
 
 value : device-resident throughput (inputs in HBM), CUDA events, max over ranks.
 e2e   : the same step through the host-buffer API (deepviewagg_b200.host_api): pinned host inputs
@@ -78,7 +82,10 @@ def parse():
     p.add_argument("--dtype", default="f32", choices=["f32", "bf16"])
     p.add_argument("--idx", default="randperm", choices=["randperm", "arange", "none"])
     p.add_argument("--counts", default="uniform", choices=["uniform", "ragged"])
-    p.add_argument("--rounds", type=int, default=0, help="timed repetitions of the K-step region (0 = from a 2.5 s budget)")
+    p.add_argument("--rounds", type=int, default=1, help="timed repetitions of the K-step region, median reported "
+                                                         "(0 = from a 2.5 s budget)")
+    p.add_argument("--dump-outputs", default="", metavar="DIR", help="write the outputs of the last timed step as "
+                                                                      "DIR/<name>.npy (float32, sampled rows)")
     p.add_argument("--sweep", default="", help="comma list of views per point (BASELINE config #5: 8,16,32,64): extra "
                                                "device-resident measurements under roofline_detail.sweep")
     p.add_argument("--no-variant-b", action="store_true", help="skip the variant-B side measurement (QKVBimodalCSRPool: scores "
@@ -293,6 +300,24 @@ def workload_config(args, world):
             "l2": "inputs (>16 GB per step) exceed the 126 MB L2; no explicit flush needed"}
 
 
+DUMP_BYTES_PER_ARRAY = 16 << 20      # four arrays: at most 64 MB per dump
+
+
+def dump_outputs(out_dir, arrays):
+    """Write each [rows, cols] device array as out_dir/<name>.npy in float32.  An array larger than
+    DUMP_BYTES_PER_ARRAY is replaced by a sample of its rows: the first rows of a seeded permutation,
+    in ascending order, so the same shape always samples the same rows."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        t = t.reshape(t.shape[0], -1)
+        keep = max(1, DUMP_BYTES_PER_ARRAY // (4 * t.shape[1]))
+        if t.shape[0] > keep:
+            rows = torch.randperm(t.shape[0], generator=torch.Generator().manual_seed(0))[:keep].sort().values
+            t = t[rows.to(t.device)]
+        np.save(os.path.join(out_dir, name + ".npy"), t.float().cpu().numpy())
+
+
 def ncu_traffic(args):
     """DRAM bytes per launch measured by ncu for this exact workload (profiles/ncu_traffic.json), or {}."""
     key = (f"points={args.points} views={args.views} channels={args.channels} groups={args.groups} "
@@ -403,18 +428,20 @@ def main():
     torch.cuda.synchronize()
 
     K = args.steps
-    # one measurement = exactly K steps; rounds sized so that the timed regions total >= 2.5 s
+    # one measurement = exactly K steps; --rounds 0 sizes the rounds so that the timed regions total >= 2.5 s
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    e0.record()
-    for _ in range(K):
-        step()
-    drain()
-    e1.record()
-    torch.cuda.synchronize()
-    probe_ms = torch.tensor([e0.elapsed_time(e1)], device=dev, dtype=torch.float64)
-    if dist is not None:
-        dist.all_reduce(probe_ms, op=dist.ReduceOp.MAX)
-    rounds = args.rounds if args.rounds > 0 else int(min(40, max(3, -(-2500.0 // float(probe_ms.item())))))
+    rounds = args.rounds
+    if rounds <= 0:
+        e0.record()
+        for _ in range(K):
+            step()
+        drain()
+        e1.record()
+        torch.cuda.synchronize()
+        probe_ms = torch.tensor([e0.elapsed_time(e1)], device=dev, dtype=torch.float64)
+        if dist is not None:
+            dist.all_reduce(probe_ms, op=dist.ReduceOp.MAX)
+        rounds = int(min(40, max(3, -(-2500.0 // float(probe_ms.item())))))
 
     sampler = ClockSampler(list(range(int(os.environ.get("LOCAL_WORLD_SIZE", str(world))))) if world > 1
                            else [local]) if rank == 0 else None
@@ -454,6 +481,8 @@ def main():
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
         round_ms.append(float(t.item()))
     clocks = sampler.stop() if sampler is not None else None
+    if rank == 0 and args.dump_outputs:       # before the side measurements reuse the plan's buffers
+        dump_outputs(args.dump_outputs, {"out": plan.out, "gx": plan.gx, "gcompat": plan.gcompat, "ggate": plan.ggate})
     pts = torch.tensor([float(N)], device=dev, dtype=torch.float64)
     if dist is not None:
         dist.all_reduce(pts, op=dist.ReduceOp.SUM)

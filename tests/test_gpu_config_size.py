@@ -8,7 +8,8 @@ was 60 000 points x 3 views; the 1 M test is property-only).
 Both the fused operator (ops.view_attention: forward, attentions, every gradient) and the whole
 GroupBimodalCSRPool module (DeepSetFeat map encoder, E_mod, E_score, gating; forward + gradients of
 inputs and of every parameter, train-mode BatchNorm over all rows) are compared with the CPU oracle
-(oracle/pooling_oracle.py, pinned on reference-executed fixtures) on the same seeded inputs.
+(oracle/pooling_oracle.py, pinned on reference-executed fixtures; run in fp64 for the module) on the same
+seeded inputs.
 Tolerance: 1e-4 relative (north_star) for fp32; storage precision for bf16, stated below."""
 import pytest
 import torch
@@ -64,14 +65,17 @@ def test_group_pool_module_at_config_size(cfg):
     x_map = torch.rand(V, 8, generator=gen)
     w = torch.randn(N, C, generator=gen)
 
-    # oracle (CPU, fp32): parameters as leaves
-    leaves = {k: v.clone().requires_grad_(True) for k, v in sd.items() if v.is_floating_point() and "running" not in k}
-    sd_o = {**sd, **leaves}
-    xo, mo = x_mod.clone().requires_grad_(True), x_map.clone().requires_grad_(True)
+    # oracle (CPU, fp64, on the same fp32 inputs): parameters as leaves.  torch's fp32 CPU batch_norm is off by
+    # ~1.6e-5 relative over a million rows (its mean and var alone are good to 1e-7); that alone puts hundreds of
+    # rows of an fp32 oracle's x_mod gradient past the bound below, so in fp64 the comparison measures the kernels.
+    sd64 = {k: v.double() if v.is_floating_point() else v for k, v in sd.items()}
+    leaves = {k: v.clone().requires_grad_(True) for k, v in sd64.items() if v.is_floating_point() and "running" not in k}
+    sd_o = {**sd64, **leaves}
+    xo, mo = x_mod.double().requires_grad_(True), x_map.double().requires_grad_(True)
     ref = O.group_pool(sd_o, xo, mo, ptr, G, use_mod=False, gating_on=True, group_scaling=True,
                        map_encoder_name="DeepSetFeat", training=True, use_num=True)
     names = list(leaves)
-    ref_g = torch.autograd.grad((ref["out"] * w).sum(), [xo, mo] + [leaves[k] for k in names], allow_unused=True)
+    ref_g = torch.autograd.grad((ref["out"] * w.double()).sum(), [xo, mo] + [leaves[k] for k in names], allow_unused=True)
 
     m = m.cuda().train()
     xg, mg = x_mod.cuda().requires_grad_(True), x_map.cuda().requires_grad_(True)
