@@ -1,7 +1,6 @@
 // C ABI of the projection GEMMs of the pool MLPs: dispatch between the skinny mma.sync kernels
 // (skinny_gemm.cu: K, N <= 64) and the hand-written tcgen05 kernels (tc_gemm.cu: everything wider).
 #include "dva_common.cuh"
-#include <stdlib.h>
 
 extern "C" int dva_skinny_gemm_supported(int64_t M, int64_t N, int64_t K, int layout);
 extern "C" size_t dva_skinny_gemm_workspace_bytes(int64_t M, int64_t N, int64_t K, int layout);
@@ -24,16 +23,10 @@ using namespace dva;
 // exceed 32 and are multiples of 4; dW (layout 2) likewise since the tcgen05 dW kernel packs its stages (round 2).
 // Round 2: the 32-wide rows GEMMs (N >= 32, K >= 8) go to the tcgen05 kernel too -- on a par as plain GEMMs, but
 // the BatchNorm statistics then come out of its epilogue (module step 6.06 -> 5.92 ms at the S3DIS shape).
-// DVA_TC_NARROW=0 (A/B knob, read once) restores the round-1 routing.
-extern "C" int dva_tc_narrow() {
-  static const int v = [] { const char* e = getenv("DVA_TC_NARROW"); return (e && e[0] == '0') ? 0 : 1; }();
-  return v;
-}
 static bool use_skinny(int64_t M, int64_t N, int64_t K, int layout) {
   if (!dva_skinny_gemm_supported(M, N, K, layout)) return false;
   if (layout == 2) return !(N > 32 && K > 32 && N % 4 == 0 && K % 4 == 0);   // 64 x 64: 2 x 155 us here, tcgen05 dW below that
-  if (dva_tc_narrow()) return !(N >= 32 && K >= 8 && N % 4 == 0 && K % 4 == 0);
-  return !(N > 32 && K > 32 && N % 4 == 0 && K % 4 == 0);
+  return !(N >= 32 && K >= 8 && N % 4 == 0 && K % 4 == 0);
 }
 
 static bool gemm_shape_ok(int64_t M, int64_t N, int64_t K) {

@@ -23,20 +23,6 @@ constexpr int kMlRows = 16;          // rows per warp tile (one m16 block of dX,
 constexpr int kMlNP = 36;            // stride of the dA -> dz tile and of the z tile (32 columns + 4: row fragments conflict-free)
 constexpr int kMlN = 32;             // widest layer output served here
 
-__device__ __forceinline__ uint32_t ml_tf32(float x) {
-  uint32_t r;
-  asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(r) : "f"(x));
-  return r;
-}
-__device__ __forceinline__ void ml_mma(float (&c)[4], const uint32_t (&a)[4], uint32_t b0, uint32_t b1) {
-  asm volatile("mma.sync.aligned.m16n8k8.row.col.f32.tf32.tf32.f32 {%0,%1,%2,%3}, {%4,%5,%6,%7}, {%8,%9}, {%0,%1,%2,%3};"
-               : "+f"(c[0]), "+f"(c[1]), "+f"(c[2]), "+f"(c[3])
-               : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(b0), "r"(b1));
-}
-__device__ __forceinline__ void ml_cp16(uint32_t dst, const float* src, bool in) {
-  asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;" ::"r"(dst), "l"(src), "r"(in ? 16 : 0) : "memory");
-}
-
 struct MlParams {
   const float *dA, *Z, *X, *W, *gamma, *beta, *mean, *invstd, *sums;
   float *dX, *partial;
@@ -59,9 +45,9 @@ mlp_layer_bwd_kernel(const MlParams p) {
   for (int e = threadIdx.x; e < kMlN * KP; e += blockDim.x) {
     const int n = e / KP, k = e - n * KP;
     const float v = (n < N && k < K) ? __ldg(p.W + (int64_t)n * K + k) : 0.f;
-    const uint32_t hi = ml_tf32(v);
+    const uint32_t hi = to_tf32(v);
     wHi[e] = hi;
-    wLo[e] = ml_tf32(v - __uint_as_float(hi));
+    wLo[e] = to_tf32(v - __uint_as_float(hi));
   }
   for (int c = threadIdx.x; c < kMlN; c += blockDim.x) {
     float sc = 0.f, sh = 0.f, mu = 0.f, is = 0.f, k0 = 0.f, k1 = 0.f;
@@ -100,21 +86,22 @@ mlp_layer_bwd_kernel(const MlParams p) {
   constexpr int XH = (NT + 3) / 4;                   // 8-chunk column blocks of x: 2 for K > 32
   auto load = [&](float* buf, int64_t t) {
     const int64_t row0 = t * kMlRows;
-    const uint32_t s0 = (uint32_t)__cvta_generic_to_shared(buf);
+    const uint32_t s0 = smem_u32(buf);
 #pragma unroll
     for (int i = 0; i < 4; ++i) {
       const int r = rr + 4 * i;
       const bool in = row0 + r < p.M;
       if (c4 < nc4) {
         const int64_t off = in ? (row0 + r) * N + c4 * 4 : 0;
-        ml_cp16(s0 + (uint32_t)(r * kMlNP + c4 * 4) * 4, p.dA + off, in);
-        ml_cp16(s0 + (uint32_t)(kMlRows * kMlNP + r * kMlNP + c4 * 4) * 4, p.Z + off, in);
+        cp_async16_zfill(s0 + (uint32_t)(r * kMlNP + c4 * 4) * 4, p.dA + off, in ? 16 : 0);
+        cp_async16_zfill(s0 + (uint32_t)(kMlRows * kMlNP + r * kMlNP + c4 * 4) * 4, p.Z + off, in ? 16 : 0);
       }
 #pragma unroll
       for (int h = 0; h < XH; ++h) {
         const int cx = c4 + 8 * h;
         if (cx < kc4)
-          ml_cp16(s0 + (uint32_t)(2 * kMlRows * kMlNP + r * KP + cx * 4) * 4, p.X + (in ? (row0 + r) * K + cx * 4 : 0), in);
+          cp_async16_zfill(s0 + (uint32_t)(2 * kMlRows * kMlNP + r * KP + cx * 4) * 4,
+                           p.X + (in ? (row0 + r) * K + cx * 4 : 0), in ? 16 : 0);
       }
     }
   };
@@ -128,15 +115,15 @@ mlp_layer_bwd_kernel(const MlParams p) {
       for (int q = 0; q < 4; ++q) acc_w[m][n][q] = 0.f;
 
   if (t0 < tiles_total) load(my, t0);
-  asm volatile("cp.async.commit_group;" ::: "memory");
+  cp_async_commit();
   int cur = 0;
   for (int64_t t = t0; t < tiles_total; t += tstep, cur ^= 1) {
     float* gS = my + cur * stage_floats;             // dA, then dz
     float* zS = gS + kMlRows * kMlNP;
     float* xS = zS + kMlRows * kMlNP;                // x, then the dX staging tile
     if (t + tstep < tiles_total) load(my + (cur ^ 1) * stage_floats, t + tstep);
-    asm volatile("cp.async.commit_group;" ::: "memory");
-    asm volatile("cp.async.wait_group 1;" ::: "memory");
+    cp_async_commit();
+    cp_async_wait<1>();
     __syncwarp();
     const int64_t row0 = t * kMlRows;
     // ---- dz in place of dA: 16 x 32 elements, one float4 per lane and step -------------------------------
@@ -173,8 +160,8 @@ mlp_layer_bwd_kernel(const MlParams p) {
           uint32_t ahi[4], alo[4];
 #pragma unroll
           for (int q = 0; q < 4; ++q) {
-            ahi[q] = ml_tf32(v[q]);
-            alo[q] = ml_tf32(v[q] - __uint_as_float(ahi[q]));
+            ahi[q] = to_tf32(v[q]);
+            alo[q] = to_tf32(v[q] - __uint_as_float(ahi[q]));
           }
           const uint32_t* bh = wHi + (ks * 8 + tq) * KP + g;
           const uint32_t* bl = wLo + (ks * 8 + tq) * KP + g;
@@ -187,11 +174,11 @@ mlp_layer_bwd_kernel(const MlParams p) {
           // the three products of one output block depend on each other through its accumulator: small terms
           // first, dependent MMAs NT apart
 #pragma unroll
-          for (int j = 0; j < NT; ++j) ml_mma(acc_x[j], alo, h0[j], h1[j]);
+          for (int j = 0; j < NT; ++j) mma_tf32(acc_x[j], alo, h0[j], h1[j]);
 #pragma unroll
-          for (int j = 0; j < NT; ++j) ml_mma(acc_x[j], ahi, l0[j], l1[j]);
+          for (int j = 0; j < NT; ++j) mma_tf32(acc_x[j], ahi, l0[j], l1[j]);
 #pragma unroll
-          for (int j = 0; j < NT; ++j) ml_mma(acc_x[j], ahi, h0[j], h1[j]);
+          for (int j = 0; j < NT; ++j) mma_tf32(acc_x[j], ahi, h0[j], h1[j]);
         }
       }
     }
@@ -206,21 +193,21 @@ mlp_layer_bwd_kernel(const MlParams p) {
         const float v[4] = {ap[m * 16], ap[m * 16 + 8], ap[4 * kMlNP + m * 16], ap[4 * kMlNP + m * 16 + 8]};
 #pragma unroll
         for (int q = 0; q < 4; ++q) {
-          ahi[m][q] = ml_tf32(v[q]);
-          alo[m][q] = ml_tf32(v[q] - __uint_as_float(ahi[m][q]));
+          ahi[m][q] = to_tf32(v[q]);
+          alo[m][q] = to_tf32(v[q] - __uint_as_float(ahi[m][q]));
         }
       }
 #pragma unroll
       for (int j = 0; j < NT; ++j) {
         const float w0 = bp[j * 8], w1 = bp[4 * KP + j * 8];
-        const uint32_t h0 = ml_tf32(w0), h1 = ml_tf32(w1);
-        const uint32_t l0 = ml_tf32(w0 - __uint_as_float(h0)), l1 = ml_tf32(w1 - __uint_as_float(h1));
+        const uint32_t h0 = to_tf32(w0), h1 = to_tf32(w1);
+        const uint32_t l0 = to_tf32(w0 - __uint_as_float(h0)), l1 = to_tf32(w1 - __uint_as_float(h1));
 #pragma unroll
-        for (int m = 0; m < 2; ++m) ml_mma(acc_w[m][j], alo[m], h0, h1);
+        for (int m = 0; m < 2; ++m) mma_tf32(acc_w[m][j], alo[m], h0, h1);
 #pragma unroll
-        for (int m = 0; m < 2; ++m) ml_mma(acc_w[m][j], ahi[m], l0, l1);
+        for (int m = 0; m < 2; ++m) mma_tf32(acc_w[m][j], ahi[m], l0, l1);
 #pragma unroll
-        for (int m = 0; m < 2; ++m) ml_mma(acc_w[m][j], ahi[m], h0, h1);
+        for (int m = 0; m < 2; ++m) mma_tf32(acc_w[m][j], ahi[m], h0, h1);
       }
     }
     // ---- dX tile through the (dead) x tile: coalesced 16-byte stores ----------------------------------------
@@ -246,7 +233,7 @@ mlp_layer_bwd_kernel(const MlParams p) {
     }
     __syncwarp();                                    // the stage may be refilled two iterations from now
   }
-  asm volatile("cp.async.wait_group 0;" ::: "memory");
+  cp_async_wait<0>();
   __syncthreads();                                   // every warp is out of its loop: the tiles become rS [4][32][NT*8]
   constexpr int OW = NT * 8;
   float* rS = tiles;

@@ -1,17 +1,13 @@
 // Skinny projections of the pool MLPs (base_modules.py:42 -- Linear(bias=False) inside every MLP
 // layer of DeepSetFeat / E_mod / E_mix, pooling.py:239-261, 645-656): [rows, K] x [N, K]^T with
-// K, N <= 64 and millions of rows (one per view).  2*K*N flops against 4*(K+N) bytes per row is
-// ~16 flop/byte at K = N = 32: HBM-bound on the fp32 pipes already, and far too narrow for the
-// 128x64 tcgen05 tiles of mlp_gemm.cu (measured there: 0.50 ms per launch at 1.28 M x 32 x 32,
-// 10x the HBM time).  Exact fp32 FFMA, weights resident in shared memory, every global access a
-// coalesced 16-byte vector through a shared staging tile:
-//   layouts 0/1  skinny_rows_mma_kernel : D[M,OUT] = A[M,RED] . Wt[RED,OUT] on mma.sync with 3xTF32
-//                split operands (fp32-grade accuracy); skinny_rows_kernel: the same on the fp32
-//                pipes, 8x8 register tiles (kept for 64 x 64 layers and as DVA_SKINNY=ffma)
-//   layout  2    skinny_dw_kernel   : D[N,K]   = A[M,N]^T . B[M,K]        (4x4 micro-tiles per
-//                thread, rows split over thread slices, per-CTA partials reduced in a fixed order)
+// K, N <= 64 and millions of rows (one per view).  linear_api.cu sends here the shapes the tcgen05
+// kernels of tc_gemm.cu do not take: odd widths, K < 8 or N < 32, and dW unless both widths exceed 32.
+// 3xTF32 split operands on mma.sync (fp32-grade accuracy), weights resident in shared memory, every
+// global access a coalesced 16-byte vector through a shared staging tile:
+//   layouts 0/1  skinny_rows_mma_kernel : D[M,OUT] = A[M,RED] . Wt[RED,OUT]
+//   layout  2    skinny_dw_mma_kernel   : D[N,K]   = A[M,N]^T . B[M,K]   (the rows are the MMA k
+//                dimension; per-CTA partials reduced in a fixed order by skinny_dw_reduce_cols_kernel)
 #include "dva_common.cuh"
-#include <stdlib.h>
 
 namespace dva {
 
@@ -26,14 +22,14 @@ __device__ __forceinline__ void sk_load_tile(float* __restrict__ dst, int dst_st
   const int nthreads = blockDim.x;
   if (vec) {
     const int c4 = cols >> 2;
-    const uint32_t d0 = (uint32_t)__cvta_generic_to_shared(dst);
+    const uint32_t d0 = smem_u32(dst);
     if (nthreads % c4 == 0) {                        // the usual case: a thread keeps its column, rows advance by a constant
       const int c = ((int)threadIdx.x % c4) << 2, rstep = nthreads / c4;
       for (int r = threadIdx.x / c4; r < kSkTile; r += rstep) {
         const bool in = row0 + r < M;
         const float* g = src + (in ? (row0 + r) * cols + c : 0);
         const int bytes = in ? 16 : 0;               // src-size 0: the 16 destination bytes are zero-filled
-        asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;" ::"r"(d0 + (uint32_t)(r * dst_stride + c) * 4), "l"(g), "r"(bytes) : "memory");
+        cp_async16_zfill(d0 + (uint32_t)(r * dst_stride + c) * 4, g, bytes);
       }
     } else {
       for (int e = threadIdx.x; e < kSkTile * c4; e += nthreads) {
@@ -41,7 +37,7 @@ __device__ __forceinline__ void sk_load_tile(float* __restrict__ dst, int dst_st
         const bool in = row0 + r < M;
         const float* g = src + (in ? (row0 + r) * cols + c : 0);
         const int bytes = in ? 16 : 0;
-        asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;" ::"r"(d0 + (uint32_t)(r * dst_stride + c) * 4), "l"(g), "r"(bytes) : "memory");
+        cp_async16_zfill(d0 + (uint32_t)(r * dst_stride + c) * 4, g, bytes);
       }
     }
   } else {
@@ -51,127 +47,15 @@ __device__ __forceinline__ void sk_load_tile(float* __restrict__ dst, int dst_st
     }
   }
 }
-__device__ __forceinline__ void sk_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
-template <int N> __device__ __forceinline__ void sk_wait() { asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory"); }
-
-// D[M,OUT] = A[M,RED] . Wt[RED,OUT].  W is given as [OUT,RED] (TRANS: layout 0, x . W^T) or as
-// [RED,OUT] (layout 1, dz . W).  A CTA tile is 128 rows; thread (rg, cg) owns an 8 x 8 register
-// tile: rows rg + 16 i (i < 8; the interleave keeps the A-tile LDS.128 conflict-free) x columns
-// 8 cg .. 8 cg + 7.  Per k that is 2 + 2 LDS.128 for 64 FFMA -- with one row per thread the
-// weights alone cost 8 LDS.128 per 32 FFMA and the kernel ran at the shared-memory bandwidth.
-template <bool TRANS>
-__global__ void __launch_bounds__(128)
-skinny_rows_kernel(const float* __restrict__ A, const float* __restrict__ W, float* __restrict__ D,
-                   int64_t M, int RED, int OUT, int avec, int dvec) {
-  extern __shared__ __align__(16) float sk_smem[];
-  const int RED4 = (RED + 3) & ~3;
-  const int REDP = RED4 + 4;                        // tile strides: multiples of 4, /4 odd -> LDS.128 conflict-free
-  const int OUTP = (OUT + 31) & ~31;                // weight tile width (zero padded)
-  const int OUTS = OUTP + 4;
-  float* wS = sk_smem;                               // [RED4][OUTP]
-  const int tile_floats = kSkTile * (REDP > OUTS ? REDP : OUTS);
-  float* tbuf = wS + RED4 * OUTP;                    // 2 x (A tile [kSkTile][REDP], later the output tile [kSkTile][OUTS])
-  for (int e = threadIdx.x; e < RED4 * OUTP; e += blockDim.x) {
-    const int k = e / OUTP, n = e - k * OUTP;
-    float v = 0.f;
-    if (k < RED && n < OUT) v = TRANS ? __ldg(W + (int64_t)n * RED + k) : __ldg(W + (int64_t)k * OUT + n);
-    wS[e] = v;
-  }
-  const int ncg = OUTP >> 3;                         // column groups of 8: 4 or 8
-  const int cg = threadIdx.x % ncg, rg = threadIdx.x / ncg;   // rg < 16
-  const int64_t tiles = (M + kSkTile - 1) / kSkTile;
-  // tile i of this CTA lives in buffer i & 1; tile i + 1 is copied in while tile i is computed
-  if (blockIdx.x < tiles) sk_load_tile(tbuf, REDP, A, (int64_t)blockIdx.x * kSkTile, M, RED, avec != 0);
-  sk_commit();
-  int cur = 0;
-  for (int64_t t = blockIdx.x; t < tiles; t += gridDim.x, cur ^= 1) {
-    const int64_t row0 = t * kSkTile;
-    float* tS = tbuf + cur * tile_floats;
-    __syncthreads();                                 // the other buffer's output has been stored
-    if (t + gridDim.x < tiles)
-      sk_load_tile(tbuf + (cur ^ 1) * tile_floats, REDP, A, (t + gridDim.x) * kSkTile, M, RED, avec != 0);
-    sk_commit();
-    sk_wait<1>();                                    // tile t has landed
-    if (RED4 != RED) {                               // zero the padding columns read by the float4 loop
-      for (int e = threadIdx.x; e < kSkTile * (RED4 - RED); e += blockDim.x) {
-        const int r = e / (RED4 - RED), c = RED + e % (RED4 - RED);
-        tS[r * REDP + c] = 0.f;
-      }
-    }
-    __syncthreads();
-    float acc[8][8];
-#pragma unroll
-    for (int i = 0; i < 8; ++i)
-#pragma unroll
-      for (int j = 0; j < 8; ++j) acc[i][j] = 0.f;
-    const float* ar = tS + rg * REDP;
-    const float* wc = wS + cg * 8;
-    for (int k = 0; k < RED4; k += 4) {
-      float4 a4[8];
-#pragma unroll
-      for (int i = 0; i < 8; ++i) a4[i] = *reinterpret_cast<const float4*>(ar + (16 * i) * REDP + k);
-#pragma unroll
-      for (int kk = 0; kk < 4; ++kk) {
-        const float4 w0 = *reinterpret_cast<const float4*>(wc + (k + kk) * OUTP);
-        const float4 w1 = *reinterpret_cast<const float4*>(wc + (k + kk) * OUTP + 4);
-#pragma unroll
-        for (int i = 0; i < 8; ++i) {
-          const float av = kk == 0 ? a4[i].x : (kk == 1 ? a4[i].y : (kk == 2 ? a4[i].z : a4[i].w));
-          acc[i][0] = fmaf(av, w0.x, acc[i][0]); acc[i][1] = fmaf(av, w0.y, acc[i][1]);
-          acc[i][2] = fmaf(av, w0.z, acc[i][2]); acc[i][3] = fmaf(av, w0.w, acc[i][3]);
-          acc[i][4] = fmaf(av, w1.x, acc[i][4]); acc[i][5] = fmaf(av, w1.y, acc[i][5]);
-          acc[i][6] = fmaf(av, w1.z, acc[i][6]); acc[i][7] = fmaf(av, w1.w, acc[i][7]);
-        }
-      }
-    }
-    __syncthreads();                                 // every thread is done reading the A tile
-#pragma unroll
-    for (int i = 0; i < 8; ++i) {
-      float* orow = tS + (rg + 16 * i) * OUTS + cg * 8;
-      *reinterpret_cast<float4*>(orow) = make_float4(acc[i][0], acc[i][1], acc[i][2], acc[i][3]);
-      *reinterpret_cast<float4*>(orow + 4) = make_float4(acc[i][4], acc[i][5], acc[i][6], acc[i][7]);
-    }
-    __syncthreads();
-    if (dvec && (int)blockDim.x % (OUT >> 2) == 0) {
-      const int c4 = OUT >> 2, c = ((int)threadIdx.x % c4) << 2, rstep = (int)blockDim.x / c4;
-      for (int r = threadIdx.x / c4; r < kSkTile; r += rstep)
-        if (row0 + r < M)
-          *reinterpret_cast<float4*>(D + (row0 + r) * OUT + c) = *reinterpret_cast<const float4*>(tS + r * OUTS + c);
-    } else if (dvec) {
-      const int c4 = OUT >> 2;
-      for (int e = threadIdx.x; e < kSkTile * c4; e += blockDim.x) {
-        const int r = e / c4, c = (e - r * c4) << 2;
-        if (row0 + r < M)
-          *reinterpret_cast<float4*>(D + (row0 + r) * OUT + c) = *reinterpret_cast<const float4*>(tS + r * OUTS + c);
-      }
-    } else {
-      for (int e = threadIdx.x; e < kSkTile * OUT; e += blockDim.x) {
-        const int r = e / OUT, c = e - r * OUT;
-        if (row0 + r < M) D[(row0 + r) * OUT + c] = tS[r * OUTS + c];
-      }
-    }
-  }
-}
 
 // ---------------------------------------------------------------------------------------------
-// Tensor-core version of the row kernel: 3xTF32 (a = a_hi + a_lo, w = w_hi + w_lo in TF32;
-// a.w ~ a_lo.w_hi + a_hi.w_lo + a_hi.w_hi accumulated in fp32 -> fp32-grade accuracy) on
-// mma.sync.m16n8k8.  4 warps per CTA, a warp owns 32 rows x all columns of the 128-row tile:
-// per k-step of 8 it loads 8 A values per lane (bank-conflict-free: tile stride = 4 mod 8 words),
-// splits them, and issues 6 MMAs per 8-column block.  ~3.8x fewer instructions than the FFMA
-// kernel, which ran at the fp32-pipe limit (61-72 % issue slots, 60-70 % of them FFMA).
+// Rows kernel: 3xTF32 (a = a_hi + a_lo, w = w_hi + w_lo in TF32; a.w ~ a_lo.w_hi + a_hi.w_lo +
+// a_hi.w_hi accumulated in fp32 -> fp32-grade accuracy) on mma.sync.m16n8k8.  4 warps per CTA, a
+// warp owns 32 rows x all columns of the 128-row tile: per k-step of 8 it loads 8 A values per lane
+// (bank-conflict-free: tile stride = 4 mod 8 words), splits them, and issues 6 MMAs per 8-column
+// block.  ~3.8x fewer instructions than the same tiles on FFMA, which ran at the fp32-pipe limit
+// (61-72 % issue slots, 60-70 % of them FFMA).
 // ---------------------------------------------------------------------------------------------
-__device__ __forceinline__ uint32_t to_tf32(float x) {
-  uint32_t r;
-  asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(r) : "f"(x));
-  return r;
-}
-__device__ __forceinline__ void mma_tf32(float (&c)[4], const uint32_t (&a)[4], uint32_t b0, uint32_t b1) {
-  asm volatile("mma.sync.aligned.m16n8k8.row.col.f32.tf32.tf32.f32 {%0,%1,%2,%3}, {%4,%5,%6,%7}, {%8,%9}, {%0,%1,%2,%3};"
-               : "+f"(c[0]), "+f"(c[1]), "+f"(c[2]), "+f"(c[3])
-               : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(b0), "r"(b1));
-}
-
 template <bool TRANS, int NT /* 8-column blocks: OUT <= 8 * NT */>
 __global__ void __launch_bounds__(128)
 skinny_rows_mma_kernel(const float* __restrict__ A, const float* __restrict__ W, float* __restrict__ D,
@@ -198,7 +82,7 @@ skinny_rows_mma_kernel(const float* __restrict__ A, const float* __restrict__ W,
   const int g = lane >> 2, tq = lane & 3;
   const int64_t tiles = (M + kSkTile - 1) / kSkTile;
   if (blockIdx.x < tiles) sk_load_tile(tbuf, REDP, A, (int64_t)blockIdx.x * kSkTile, M, RED, avec != 0);
-  sk_commit();
+  cp_async_commit();
   int cur = 0;
   for (int64_t t = blockIdx.x; t < tiles; t += gridDim.x, cur ^= 1) {
     const int64_t row0 = t * kSkTile;
@@ -207,8 +91,8 @@ skinny_rows_mma_kernel(const float* __restrict__ A, const float* __restrict__ W,
     __syncthreads();                                 // the other buffer's output has been stored
     if (t + gridDim.x < tiles)
       sk_load_tile(tbuf + (cur ^ 1) * tile_floats, REDP, A, (t + gridDim.x) * kSkTile, M, RED, avec != 0);
-    sk_commit();
-    sk_wait<1>();                                    // tile t has landed
+    cp_async_commit();
+    cp_async_wait<1>();                                    // tile t has landed
     if (RED8 != RED) {                               // padding columns of the k-loop (an output tile lived here before)
       for (int e = threadIdx.x; e < kSkTile * (RED8 - RED); e += blockDim.x) {
         const int r = e / (RED8 - RED), c = RED + e % (RED8 - RED);
@@ -311,85 +195,6 @@ static int sk_rows_mma(const float* A, const float* B, float* D, int64_t M, int 
   return sk_launch_rows_mma<TRANS, 8>(A, B, D, M, RED, OUT, st);
 }
 
-// partial[cta][N*K] = sum over the CTA's rows of A[r][n] * B[r][k].  8 x 8 micro-tiles of the
-// [N,K] result per thread (2 + 2 LDS.128 for 64 FFMA per row); the rows of a tile are split over
-// 128 / (#micro-tiles) thread slices whose partial sums meet in shared memory at the end.
-constexpr int kSkDwThreads = 128;
-__global__ void __launch_bounds__(kSkDwThreads)
-skinny_dw_kernel(const float* __restrict__ A, const float* __restrict__ B, float* __restrict__ partial,
-                 int64_t M, int N, int K, int avec, int bvec) {
-  extern __shared__ __align__(16) float sk_smem[];
-  const int N8 = (N + 7) & ~7, K8 = (K + 7) & ~7;
-  const int NP = N8 + 4, KP = K8 + 4;
-  const int pair_floats = kSkTile * (NP + KP);       // one buffer = A tile [kSkTile][NP] + B tile [kSkTile][KP]
-  float* rS = sk_smem;                               // cross-slice reduction [threads][64], after the last tile
-  const int ntk = K8 >> 3, nt = (N8 >> 3) * ntk;     // 8x8 micro-tiles: at most 64
-  const int slices = kSkDwThreads / nt;
-  const int mt = threadIdx.x % nt, slice = threadIdx.x / nt;
-  const bool worker = slice < slices;
-  const int n0 = (mt / ntk) << 3, k0 = (mt % ntk) << 3;
-  float acc[8][8];
-#pragma unroll
-  for (int i = 0; i < 8; ++i)
-#pragma unroll
-    for (int j = 0; j < 8; ++j) acc[i][j] = 0.f;
-  // padding columns stay zero for the whole kernel
-  for (int e = threadIdx.x; e < 2 * pair_floats; e += blockDim.x) sk_smem[e] = 0.f;
-  __syncthreads();
-  const int64_t tiles = (M + kSkTile - 1) / kSkTile;
-  if (blockIdx.x < tiles) {
-    sk_load_tile(sk_smem, NP, A, (int64_t)blockIdx.x * kSkTile, M, N, avec != 0);
-    sk_load_tile(sk_smem + kSkTile * NP, KP, B, (int64_t)blockIdx.x * kSkTile, M, K, bvec != 0);
-  }
-  sk_commit();
-  int cur = 0;
-  for (int64_t t = blockIdx.x; t < tiles; t += gridDim.x, cur ^= 1) {
-    const float* aS = sk_smem + cur * pair_floats;
-    const float* bS = aS + kSkTile * NP;
-    __syncthreads();                                 // every thread is done with the other buffer
-    if (t + gridDim.x < tiles) {
-      float* nx = sk_smem + (cur ^ 1) * pair_floats;
-      sk_load_tile(nx, NP, A, (t + gridDim.x) * kSkTile, M, N, avec != 0);
-      sk_load_tile(nx + kSkTile * NP, KP, B, (t + gridDim.x) * kSkTile, M, K, bvec != 0);
-    }
-    sk_commit();
-    sk_wait<1>();
-    __syncthreads();
-    if (worker) {
-#pragma unroll 2
-      for (int r = slice; r < kSkTile; r += slices) {
-        const float4 a0 = *reinterpret_cast<const float4*>(aS + r * NP + n0);
-        const float4 a1 = *reinterpret_cast<const float4*>(aS + r * NP + n0 + 4);
-        const float4 b0 = *reinterpret_cast<const float4*>(bS + r * KP + k0);
-        const float4 b1 = *reinterpret_cast<const float4*>(bS + r * KP + k0 + 4);
-        const float av[8] = {a0.x, a0.y, a0.z, a0.w, a1.x, a1.y, a1.z, a1.w};
-#pragma unroll
-        for (int i = 0; i < 8; ++i) {
-          acc[i][0] = fmaf(av[i], b0.x, acc[i][0]); acc[i][1] = fmaf(av[i], b0.y, acc[i][1]);
-          acc[i][2] = fmaf(av[i], b0.z, acc[i][2]); acc[i][3] = fmaf(av[i], b0.w, acc[i][3]);
-          acc[i][4] = fmaf(av[i], b1.x, acc[i][4]); acc[i][5] = fmaf(av[i], b1.y, acc[i][5]);
-          acc[i][6] = fmaf(av[i], b1.z, acc[i][6]); acc[i][7] = fmaf(av[i], b1.w, acc[i][7]);
-        }
-      }
-    }
-  }
-  __syncthreads();                                   // tiles are dead: their memory becomes rS
-#pragma unroll
-  for (int i = 0; i < 8; ++i)
-#pragma unroll
-    for (int j = 0; j < 8; ++j) rS[threadIdx.x * 64 + i * 8 + j] = worker ? acc[i][j] : 0.f;
-  __syncthreads();
-  // slices summed in a fixed order; micro-tile (n0,k0) element (i,j) -> partial[n0+i][k0+j]
-  float* out = partial + (int64_t)blockIdx.x * N * K;
-  for (int e = threadIdx.x; e < nt * 64; e += blockDim.x) {
-    const int m = e >> 6, ij = e & 63;
-    float sum = 0.f;
-    for (int sl = 0; sl < slices; ++sl) sum += rS[(sl * nt + m) * 64 + ij];
-    const int n = ((m / ntk) << 3) + (ij >> 3), k = ((m % ntk) << 3) + (ij & 7);
-    if (n < N && k < K) out[n * K + k] = sum;
-  }
-}
-
 // ---------------------------------------------------------------------------------------------
 // Tensor-core dW: partial[cta][N x kcols] = sum_rows A[r][n] * B[r][kofs + k] with the ROWS as the
 // MMA k-dimension (m16n8k8: m = 16 outputs n, n = 8 outputs k, k = 8 rows), 3xTF32 split operands.
@@ -419,22 +224,20 @@ skinny_dw_mma_kernel(const float* __restrict__ A, const float* __restrict__ B, f
   __syncthreads();
   // tile loader: 64 rows of A (N columns) and of B (kcols columns starting at kofs)
   auto load = [&](float* buf, int64_t row0) {
-    const uint32_t a0 = (uint32_t)__cvta_generic_to_shared(buf), b0 = a0 + kSkDwRows * NP * 4;
+    const uint32_t a0 = smem_u32(buf), b0 = a0 + kSkDwRows * NP * 4;
     if (avec) {
       const int c4 = N >> 2;
       if ((int)blockDim.x % c4 == 0) {               // the usual widths: a thread keeps its chunk, rows advance by a constant (no division in the loop)
         const int c = ((int)threadIdx.x % c4) << 2, rstep = (int)blockDim.x / c4;
         for (int r = threadIdx.x / c4; r < kSkDwRows; r += rstep) {
           const bool in = row0 + r < M;
-          asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;" ::"r"(a0 + (uint32_t)(r * NP + c) * 4),
-                       "l"(A + (in ? (row0 + r) * N + c : 0)), "r"(in ? 16 : 0) : "memory");
+          cp_async16_zfill(a0 + (uint32_t)(r * NP + c) * 4, A + (in ? (row0 + r) * N + c : 0), in ? 16 : 0);
         }
       } else {
         for (int e = threadIdx.x; e < kSkDwRows * c4; e += blockDim.x) {
           const int r = e / c4, c = (e - r * c4) << 2;
           const bool in = row0 + r < M;
-          asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;" ::"r"(a0 + (uint32_t)(r * NP + c) * 4),
-                       "l"(A + (in ? (row0 + r) * N + c : 0)), "r"(in ? 16 : 0) : "memory");
+          cp_async16_zfill(a0 + (uint32_t)(r * NP + c) * 4, A + (in ? (row0 + r) * N + c : 0), in ? 16 : 0);
         }
       }
     } else {
@@ -450,15 +253,13 @@ skinny_dw_mma_kernel(const float* __restrict__ A, const float* __restrict__ B, f
         const int c = ((int)threadIdx.x % c4) << 2, rstep = (int)blockDim.x / c4;
         for (int r = threadIdx.x / c4; r < kSkDwRows; r += rstep) {
           const bool in = row0 + r < M;
-          asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;" ::"r"(b0 + (uint32_t)(r * KP + c) * 4),
-                       "l"(B + (in ? (row0 + r) * K + kofs + c : 0)), "r"(in ? 16 : 0) : "memory");
+          cp_async16_zfill(b0 + (uint32_t)(r * KP + c) * 4, B + (in ? (row0 + r) * K + kofs + c : 0), in ? 16 : 0);
         }
       } else {
         for (int e = threadIdx.x; e < kSkDwRows * c4; e += blockDim.x) {
           const int r = e / c4, c = (e - r * c4) << 2;
           const bool in = row0 + r < M;
-          asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;" ::"r"(b0 + (uint32_t)(r * KP + c) * 4),
-                       "l"(B + (in ? (row0 + r) * K + kofs + c : 0)), "r"(in ? 16 : 0) : "memory");
+          cp_async16_zfill(b0 + (uint32_t)(r * KP + c) * 4, B + (in ? (row0 + r) * K + kofs + c : 0), in ? 16 : 0);
         }
       }
     } else {
@@ -470,15 +271,15 @@ skinny_dw_mma_kernel(const float* __restrict__ A, const float* __restrict__ B, f
   };
   const int64_t tiles = (M + kSkDwRows - 1) / kSkDwRows;
   if (blockIdx.x < tiles) load(sk_smem, (int64_t)blockIdx.x * kSkDwRows);
-  sk_commit();
+  cp_async_commit();
   int cur = 0;
   for (int64_t t = blockIdx.x; t < tiles; t += gridDim.x, cur ^= 1) {
     const float* aS = sk_smem + cur * pair_floats;
     const float* bS = aS + kSkDwRows * NP;
     __syncthreads();                                 // every warp is done with the other buffer
     if (t + gridDim.x < tiles) load(sk_smem + (cur ^ 1) * pair_floats, (t + gridDim.x) * kSkDwRows);
-    sk_commit();
-    sk_wait<1>();
+    cp_async_commit();
+    cp_async_wait<1>();
     __syncthreads();
 #pragma unroll
     for (int ks = 0; ks < 2; ++ks) {                 // this warp's 16 rows = two k-steps of 8 rows
@@ -555,26 +356,6 @@ skinny_dw_reduce_cols_kernel(const float* __restrict__ partial, float* __restric
   if (lane == 0) D[(e / kcols) * K + kofs + e % kcols] = s;
 }
 
-// D[e] = sum_cta partial[cta][e]: one warp per element, lanes stride over the CTAs (coalesced
-// across the warps of a block), fixed-order butterfly at the end -> deterministic
-__global__ void __launch_bounds__(256)
-skinny_dw_reduce_kernel(const float* __restrict__ partial, float* __restrict__ D, int ctas, int NK) {
-  const int lane = threadIdx.x & 31;
-  const int e = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
-  if (e >= NK) return;
-  float s = 0.f;
-  for (int c = lane; c < ctas; c += 32) s += partial[(int64_t)c * NK + e];
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
-  if (lane == 0) D[e] = s;
-}
-
-static int sk_dw_grid(int64_t M) {
-  const int64_t tiles = (M + kSkTile - 1) / kSkTile;
-  const int64_t cap = (int64_t)kNumSMs * 3;    // 74 KB of shared memory per CTA at N = K = 32
-  return (int)(tiles < cap ? (tiles < 1 ? 1 : tiles) : cap);
-}
-
 }  // namespace dva
 
 using namespace dva;
@@ -589,8 +370,7 @@ extern "C" size_t dva_skinny_gemm_workspace_bytes(int64_t M, int64_t N, int64_t 
   if (layout != 2) return 16;
   const int64_t t64 = (M + kSkDwRows - 1) / kSkDwRows, cap = (int64_t)kNumSMs * 4;
   const size_t ctas = (size_t)(t64 < cap ? t64 : cap);
-  const size_t a = (size_t)sk_dw_grid(M), c = a > ctas ? a : ctas;
-  return c * (size_t)N * (size_t)K * sizeof(float) + 16;
+  return ctas * (size_t)N * (size_t)K * sizeof(float) + 16;
 }
 
 // layout 0: D[M,N] = A[M,K] . B[N,K]^T;  1: D[M,N] = A[M,K] . B[K,N];  2: D[N,K] = A[M,N]^T . B[M,K]
@@ -600,76 +380,39 @@ extern "C" int dva_skinny_gemm(const float* A, const float* B, float* D, int64_t
   if (!dva_skinny_gemm_supported(M, N, K, layout)) return fail(DVA_EUNSUPPORTED, "skinny_gemm: N and K must be <= 64");
   if (!A || !B || !D) return fail(DVA_EINVAL, "skinny_gemm: null pointer");
   cudaStream_t st = (cudaStream_t)stream;
-  // DVA_SKINNY=ffma keeps the rows on the fp32 pipes (A/B knob; default: 3xTF32 tensor-core kernels)
-  static const bool use_mma = [] { const char* e = getenv("DVA_SKINNY"); return !(e && strcmp(e, "ffma") == 0); }();
-  if ((layout == 0 || layout == 1) && use_mma)
+  if (layout == 0 || layout == 1)
     return layout == 0 ? sk_rows_mma<true>(A, B, D, M, (int)K, (int)N, st) : sk_rows_mma<false>(A, B, D, M, (int)K, (int)N, st);
-  if (layout == 0 || layout == 1) {
-    const int RED = (int)K, OUT = (int)N;
-    const int RED4 = (RED + 3) & ~3, REDP = RED4 + 4, OUTP = (OUT + 31) & ~31, OUTS = OUTP + 4;
-    const int tile_floats = kSkTile * (REDP > OUTS ? REDP : OUTS);
-    const size_t smem = (size_t)(RED4 * OUTP + 2 * tile_floats) * sizeof(float);
-    const int threads = 16 * (OUTP / 8);             // 64 (OUT <= 32) or 128
-    const int avec = (RED % 4 == 0) && aligned16(A), dvec = (OUT % 4 == 0) && aligned16(D);
-    const int64_t tiles = (M + kSkTile - 1) / kSkTile;
-    const int64_t cap = (int64_t)kNumSMs * 5;    // ~41 KB per CTA at K = N = 32
-    const int grid = (int)(tiles < cap ? tiles : cap);
-    if (layout == 0) {
-      if (smem > 48 * 1024) cudaFuncSetAttribute(skinny_rows_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-      skinny_rows_kernel<true><<<grid, threads, smem, st>>>(A, B, D, M, RED, OUT, avec, dvec);
-    } else {
-      if (smem > 48 * 1024) cudaFuncSetAttribute(skinny_rows_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-      skinny_rows_kernel<false><<<grid, threads, smem, st>>>(A, B, D, M, RED, OUT, avec, dvec);
-    }
-    return check_launch("skinny_gemm(rows)");
-  }
   if (layout != 2) return fail(DVA_EINVAL, "skinny_gemm: bad layout");
-  if (use_mma) {
-    // output N x K in column blocks of at most 32 (64 when N <= 32) so that MT * NT <= 16 register tiles
-    const int MT = N <= 32 ? 2 : 4;
-    const int kblk = (MT == 2) ? 64 : 32;
-    const int64_t tiles = (M + kSkDwRows - 1) / kSkDwRows;
-    const int64_t cap = (int64_t)kNumSMs * 4;
-    const int grid = (int)(tiles < cap ? tiles : cap);
-    if (!workspace || workspace_bytes < (size_t)grid * N * K * sizeof(float))
-      return fail(DVA_EINVAL, "skinny_gemm: workspace too small");
-    float* partial = reinterpret_cast<float*>(workspace);
-    const int avec = (N % 4 == 0) && aligned16(A);
-    for (int kofs = 0; kofs < (int)K; kofs += kblk) {
-      const int kcols = ((int)K - kofs < kblk) ? (int)K - kofs : kblk;
-      const int NT = kcols <= 8 ? 1 : (kcols <= 32 ? 4 : 8);
-      const int bvec = (K % 4 == 0) && (kofs % 4 == 0) && (kcols % 4 == 0) && aligned16(B);
-      const int NP = MT * 16 + 8, KP = NT * 8 + 8;
-      size_t smem = (size_t)2 * kSkDwRows * (NP + KP) * sizeof(float);
-      const size_t red = (size_t)4 * MT * 16 * NT * 8 * sizeof(float);
-      if (smem < red) smem = red;
-#define SK_DW(MTv, NTv)                                                                            \
-      do {                                                                                         \
-        auto kern = skinny_dw_mma_kernel<MTv, NTv>;                                                \
-        if (smem > 48 * 1024) cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem); \
-        kern<<<grid, 128, smem, st>>>(A, B, partial, M, (int)N, (int)K, kofs, kcols, avec, bvec);  \
-      } while (0)
-      if (MT == 2) { if (NT == 1) SK_DW(2, 1); else if (NT == 4) SK_DW(2, 4); else SK_DW(2, 8); }
-      else { if (NT == 1) SK_DW(4, 1); else SK_DW(4, 4); }
-#undef SK_DW
-      if (int rc = check_launch("skinny_gemm(dw, 3xTF32 mma)")) return rc;
-      skinny_dw_reduce_cols_kernel<<<((int)N * kcols + 7) / 8, 256, 0, st>>>(partial, D, grid, (int)N, (int)K, kofs, kcols);
-      if (int rc = check_launch("skinny_gemm(dw reduce)")) return rc;
-    }
-    return DVA_OK;
-  }
-  const int grid = sk_dw_grid(M);
+  // output N x K in column blocks of at most 32 (64 when N <= 32) so that MT * NT <= 16 register tiles
+  const int MT = N <= 32 ? 2 : 4;
+  const int kblk = (MT == 2) ? 64 : 32;
+  const int64_t tiles = (M + kSkDwRows - 1) / kSkDwRows;
+  const int64_t cap = (int64_t)kNumSMs * 4;
+  const int grid = (int)(tiles < cap ? tiles : cap);
   if (!workspace || workspace_bytes < (size_t)grid * N * K * sizeof(float))
     return fail(DVA_EINVAL, "skinny_gemm: workspace too small");
-  const int N8 = ((int)N + 7) & ~7, K8 = ((int)K + 7) & ~7;
-  size_t smem = (size_t)2 * (kSkTile * (N8 + 4) + kSkTile * (K8 + 4)) * sizeof(float);
-  if (smem < (size_t)kSkDwThreads * 64 * sizeof(float)) smem = (size_t)kSkDwThreads * 64 * sizeof(float);
-  if (smem > 48 * 1024) cudaFuncSetAttribute(skinny_dw_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-  const int avec = (N % 4 == 0) && aligned16(A), bvec = (K % 4 == 0) && aligned16(B);
   float* partial = reinterpret_cast<float*>(workspace);
-  skinny_dw_kernel<<<grid, kSkDwThreads, smem, st>>>(A, B, partial, M, (int)N, (int)K, avec, bvec);
-  if (int rc = check_launch("skinny_gemm(dw)")) return rc;
-  const int NK = (int)(N * K);
-  skinny_dw_reduce_kernel<<<(NK + 7) / 8, 256, 0, st>>>(partial, D, grid, NK);
-  return check_launch("skinny_gemm(dw reduce)");
+  const int avec = (N % 4 == 0) && aligned16(A);
+  for (int kofs = 0; kofs < (int)K; kofs += kblk) {
+    const int kcols = ((int)K - kofs < kblk) ? (int)K - kofs : kblk;
+    const int NT = kcols <= 8 ? 1 : (kcols <= 32 ? 4 : 8);
+    const int bvec = (K % 4 == 0) && (kofs % 4 == 0) && (kcols % 4 == 0) && aligned16(B);
+    const int NP = MT * 16 + 8, KP = NT * 8 + 8;
+    size_t smem = (size_t)2 * kSkDwRows * (NP + KP) * sizeof(float);
+    const size_t red = (size_t)4 * MT * 16 * NT * 8 * sizeof(float);
+    if (smem < red) smem = red;
+#define SK_DW(MTv, NTv)                                                                            \
+    do {                                                                                           \
+      auto kern = skinny_dw_mma_kernel<MTv, NTv>;                                                  \
+      if (smem > 48 * 1024) cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem); \
+      kern<<<grid, 128, smem, st>>>(A, B, partial, M, (int)N, (int)K, kofs, kcols, avec, bvec);    \
+    } while (0)
+    if (MT == 2) { if (NT == 1) SK_DW(2, 1); else if (NT == 4) SK_DW(2, 4); else SK_DW(2, 8); }
+    else { if (NT == 1) SK_DW(4, 1); else SK_DW(4, 4); }
+#undef SK_DW
+    if (int rc = check_launch("skinny_gemm(dw, 3xTF32 mma)")) return rc;
+    skinny_dw_reduce_cols_kernel<<<((int)N * kcols + 7) / 8, 256, 0, st>>>(partial, D, grid, (int)N, (int)K, kofs, kcols);
+    if (int rc = check_launch("skinny_gemm(dw reduce)")) return rc;
+  }
+  return DVA_OK;
 }

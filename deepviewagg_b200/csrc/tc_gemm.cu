@@ -46,25 +46,9 @@ constexpr int kThreadsAll = kThreads + kSplitThreads;   // + a second set of spl
 constexpr uint32_t kTmemCols = 256;        // two 128-column accumulators
 constexpr uint32_t kTmemColsW = 512;       // + weight hi at column 256, weight lo at column 384 (K <= 128 each)
 
-// ---- PTX wrappers ------------------------------------------------------------------------------
-__device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-
-__device__ __forceinline__ void mbar_init(uint32_t bar, uint32_t count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count) : "memory");
-}
-__device__ __forceinline__ void mbar_expect_tx(uint32_t bar, uint32_t bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
-}
+// ---- PTX wrappers (tcgen05, TMA tensor copies; the generic async-copy ones are in dva_common.cuh) ----------
 __device__ __forceinline__ void mbar_arrive(uint32_t bar) {
   asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory");
-}
-__device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
-  uint32_t done;
-  do {
-    asm volatile(
-        "{ .reg .pred p; mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2; selp.u32 %0, 1, 0, p; }"
-        : "=r"(done) : "r"(bar), "r"(parity) : "memory");
-  } while (!done);
 }
 __device__ __forceinline__ void tma_load_2d(uint32_t dst, const CUtensorMap* map, int c0, int c1, uint32_t bar) {
   asm volatile(
@@ -74,7 +58,6 @@ __device__ __forceinline__ void tma_load_2d(uint32_t dst, const CUtensorMap* map
 __device__ __forceinline__ void tma_prefetch_desc(const CUtensorMap* map) {
   asm volatile("prefetch.tensormap [%0];" ::"l"(map) : "memory");
 }
-__device__ __forceinline__ void fence_proxy_async() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
 __device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
 __device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
 __device__ __forceinline__ void tmem_alloc(uint32_t dst_smem, uint32_t cols) {
@@ -224,7 +207,7 @@ tc_rows_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_constant_
     for (int s = 0; s < NS; ++s) { mbar_init(full_tma(s), 1); mbar_init(full_cvt(s), kSplitThreads / 32); mbar_init(empty(s), 1); }
     for (int a = 0; a < 2; ++a) { mbar_init(tmem_full(a), 1); mbar_init(tmem_empty(a), 4); }
     mbar_init(w_full, 4);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    fence_mbar_init();
   }
   if (warp == 1) tmem_alloc(smem_u32(tmem_slot), WTMEM ? kTmemColsW : kTmemCols);
   tc_fence_before();
@@ -489,7 +472,7 @@ tc_dw_kernel(const __grid_constant__ CUtensorMap map_dz, const __grid_constant__
     tma_prefetch_desc(&map_dz); tma_prefetch_desc(&map_x);
     for (int s = 0; s < NS; ++s) { mbar_init(full_tma(s), 1); mbar_init(full_cvt(s), kSplitThreads / 32); mbar_init(empty(s), 1); }
     mbar_init(tmem_full, 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    fence_mbar_init();
   }
   if (warp == 1) tmem_alloc(smem_u32(tmem_slot), kDwTmemCols);
   tc_fence_before();
@@ -849,11 +832,8 @@ extern "C" size_t dva_linear_bnstats_workspace_bytes(int64_t n_out, int64_t k_re
   return dva_tc_rows_workspace_bytes(n_out, k_red) + (size_t)kNumSMs * 3 * tc::kTile * 4;
 }
 
-extern "C" int dva_tc_narrow();
 extern "C" int dva_linear_bnstats_supported(int64_t M, int64_t n_out, int64_t k_red) {
-  if (!(dva_tc_rows_supported(M, n_out, k_red) && n_out <= tc::kTile && n_out % 4 == 0)) return 0;
-  if (dva_tc_narrow()) return n_out >= 32 && k_red >= 8;
-  return n_out > 32 && k_red > 32;
+  return dva_tc_rows_supported(M, n_out, k_red) && n_out <= tc::kTile && n_out % 4 == 0 && n_out >= 32 && k_red >= 8;
 }
 
 extern "C" int dva_linear_bnstats_fwd(const float* X, const float* W, float* D, int64_t M, int64_t n_out,

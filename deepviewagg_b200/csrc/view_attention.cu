@@ -683,8 +683,9 @@ template <typename T> static int bwd_typed(const VAParams& P, int* grid, cudaStr
 
 static bool pow2_le32(int64_t g) { return g >= 1 && g <= 32 && (g & (g - 1)) == 0; }
 
-// 0 = auto, 1 = streaming kernels, 2 = ring kernels (when applicable).  Process-wide tuning knob
-// (dva_view_attention_set_path / DVA_VA_PATH=auto|stream|ring, read once); results do not depend on it.
+// 0 = auto, 1 = streaming kernels, 2 = ring forward + lane backward, 3 = lane backward + streaming forward
+// (each where applicable).  Process-wide tuning knob (dva_view_attention_set_path /
+// DVA_VA_PATH=auto|stream|ring|lane, read once); results do not depend on it.
 static std::atomic<int>& va_path() {
   static std::atomic<int> p{[] {
     const char* e = getenv("DVA_VA_PATH");
@@ -697,31 +698,27 @@ static std::atomic<int>& va_path() {
   return p;
 }
 
-// auto (measured on B200, tools/bench_shapes.py, profiles/r1_shapes_*.json): the ring kernels win
-// where per-point scalar work dominates -- short segments.  Forward: fewer than
-// DVA_RING_MAX_MEAN_VIEWS views per point on average; backward: additionally rows of at most 128
-// bytes (with wider rows the streaming backward is as fast and needs no shared-memory tiles).
+// Short segments: the per-point scalar work dominates, and the ring forward / lane backward give it a
+// lane per point or per view.  Auto (measured on B200, tools/bench_shapes.py, profiles/r1_shapes_*.json,
+// profiles/r2_shapes_*.json): both need at most DVA_RING_MAX_MEAN_VIEWS views per point on average.
 #ifndef DVA_RING_MAX_MEAN_VIEWS
 #define DVA_RING_MAX_MEAN_VIEWS 12
 #endif
-static bool use_ring(const VAParams& P, int dtype, bool applicable, bool backward) {
+static bool use_ring_fwd(const VAParams& P, bool applicable) {
   if (!applicable) return false;
   const int path = va_path().load(std::memory_order_relaxed);
   if (path == 1 || path == 3) return false;
   if (path == 2) return true;
-  if (P.V > (int64_t)DVA_RING_MAX_MEAN_VIEWS * P.N) return false;
-  const size_t esz = dtype == DVA_F32 ? 4 : 2;
-  return !backward || (size_t)P.C * esz <= 128;
+  return P.V <= (int64_t)DVA_RING_MAX_MEAN_VIEWS * P.N;
 }
 
-// backward only: the lane-per-view kernel (view_attention_lane.cu) for short segments, path 3 forces it
-// auto (profiles/r2_shapes_*.json): short segments AND rows of at most 256 bytes -- with 512-byte rows the
-// streaming backward is as fast (1 M x 8 x 128: 1.85 ms vs 1.99 ms)
+// backward: the lane-per-view kernel (view_attention_lane.cu); auto also needs rows of at most 256 bytes --
+// with 512-byte rows the streaming backward is as fast (1 M x 8 x 128: 1.85 ms vs 1.99 ms)
 static bool use_lane_bwd(const VAParams& P, int dtype, bool applicable) {
   if (!applicable) return false;
   const int path = va_path().load(std::memory_order_relaxed);
-  if (path == 3) return true;
-  if (path != 0) return false;
+  if (path == 2 || path == 3) return true;
+  if (path == 1) return false;
   const size_t esz = dtype == DVA_F32 ? 4 : 2;
   return P.V <= (int64_t)DVA_RING_MAX_MEAN_VIEWS * P.N && (size_t)P.C * esz <= 256;
 }
@@ -754,7 +751,7 @@ extern "C" int dva_view_attention_fwd(const void* x, const void* idx, int idx_is
   P.N = N; P.V = V; P.R = R; P.C = (int)C; P.G = (int)G; P.group_scaling = group_scaling; P.eps = eps;
   cudaStream_t st = (cudaStream_t)stream;
   if (dtype != DVA_F32 && dtype != DVA_BF16 && dtype != DVA_F16) return fail(DVA_EINVAL, "view_attention_fwd: unknown dtype");
-  if (use_ring(P, dtype, va_ring_fwd_applicable(P, dtype), false)) return va_ring_fwd(P, dtype, st);
+  if (use_ring_fwd(P, va_ring_fwd_applicable(P, dtype))) return va_ring_fwd(P, dtype, st);
   switch (dtype) {
     case DVA_F32: return fwd_typed<float>(P, st);
     case DVA_BF16: return fwd_typed<__nv_bfloat16>(P, st);
@@ -764,7 +761,7 @@ extern "C" int dva_view_attention_fwd(const void* x, const void* idx, int idx_is
 }
 
 extern "C" int dva_view_attention_set_path(int path) {
-  if (path < 0 || path > 3) return fail(DVA_EINVAL, "view_attention_set_path: 0 = auto, 1 = streaming, 2 = ring, 3 = lane (backward)");
+  if (path < 0 || path > 3) return fail(DVA_EINVAL, "view_attention_set_path: 0 = auto, 1 = streaming, 2 = ring, 3 = lane");
   va_path().store(path, std::memory_order_relaxed);
   return DVA_OK;
 }
@@ -810,8 +807,6 @@ extern "C" int dva_view_attention_bwd(const void* x, const void* idx, int idx_is
   if (dtype != DVA_F32 && dtype != DVA_BF16 && dtype != DVA_F16) return fail(DVA_EINVAL, "view_attention_bwd: unknown dtype");
   if (use_lane_bwd(P, dtype, va_lane_bwd_applicable(P, dtype))) {
     rc = va_lane_bwd(P, dtype, &grid, st);
-  } else if (use_ring(P, dtype, va_ring_bwd_applicable(P, dtype), true)) {
-    rc = va_ring_bwd(P, dtype, &grid, st);
   } else {
     switch (dtype) {
       case DVA_F32: rc = bwd_typed<float>(P, &grid, st); break;

@@ -1,9 +1,10 @@
-// Shared between the two implementations of the fused view-attention pair:
-//   view_attention.cu       streaming kernels (row chunks live in registers; best for long segments
-//                           of >= 512-byte rows)
-//   view_attention_ring.cu  ring kernels (rows staged in shared memory by cp.async / bulk copies,
-//                           several batches in flight per warp across point boundaries; best for
-//                           short segments and rows <= 512 bytes)
+// Shared between the kernels of the fused view-attention pair:
+//   view_attention.cu       streaming forward and backward (row chunks live in registers, one point
+//                           per warp at a time; best for long segments and >= 512-byte rows)
+//   view_attention_ring.cu  ring forward (rows staged in shared memory by cp.async, several batches
+//                           in flight per warp across point boundaries; short segments, rows <= 512 bytes)
+//   view_attention_lane.cu  lane-per-view backward (groups of <= 32 views per warp, rows by bulk async
+//                           copies; short segments, rows <= 512 bytes)
 #pragma once
 #include "dva_common.cuh"
 
@@ -31,14 +32,17 @@ __device__ __forceinline__ float group_lane_sum(float v, int G) {
   return v;
 }
 
-// ring path (view_attention_ring.cu).  *_applicable: shape / alignment conditions of the ring
-// kernels; the launchers return a DVA_* / cudaError code like every other entry point.
-bool va_ring_fwd_applicable(const VAParams& P, int dtype);
-bool va_ring_bwd_applicable(const VAParams& P, int dtype);
-int va_ring_fwd(const VAParams& P, int dtype, cudaStream_t st);
-int va_ring_bwd(const VAParams& P, int dtype, int* grid_out, cudaStream_t st);
+// row of x of view v: idx[v] (int32 or int64 idx) or v itself; callers check V < 2^31, R < 2^32
+__device__ __forceinline__ uint32_t load_row_id(const void* idx, int idx64, int64_t v) {
+  if (idx == nullptr) return (uint32_t)v;
+  return idx64 ? (uint32_t) reinterpret_cast<const int64_t*>(idx)[v]
+               : (uint32_t) reinterpret_cast<const int32_t*>(idx)[v];
+}
 
-// lane-per-view backward for short segments (view_attention_lane.cu)
+// *_applicable: shape / alignment conditions of the ring forward and the lane backward; the launchers
+// return a DVA_* / cudaError code like every other entry point.
+bool va_ring_fwd_applicable(const VAParams& P, int dtype);
+int va_ring_fwd(const VAParams& P, int dtype, cudaStream_t st);
 bool va_lane_bwd_applicable(const VAParams& P, int dtype);
 int va_lane_bwd(const VAParams& P, int dtype, int* grid_out, cudaStream_t st);
 

@@ -1,13 +1,14 @@
 // "Lane per view" backward of the fused view-attention pair for SHORT segments (the shapes every shipped
 // config runs: S3DIS / ScanNet ~7 views per point, rows of 128 .. 512 bytes).  Same math and C ABI as
 // view_attention.cu (reference chain: modules.py:518 row gather -> pooling.py:285-300 / 515-530, gradients
-// SURVEY.md Appendix A); third implementation next to the streaming and the ring kernels.
+// SURVEY.md Appendix A); the short-segment backward next to the streaming kernels and the ring forward.
 //
 // Why.  ncu at the S3DIS step shape: the streaming backward spends a whole warp on one point at a time
-// (836 warp instructions per point, issue-bound), the ring backward halves the instruction count but its
-// 29 KB of shared memory per warp leave 8 warps per SM (21 % issue-active, latency-bound): 0.47 of the HBM
-// peak.  Here a warp takes a GROUP of consecutive points holding at most 32 views and gives every kind of
-// work its natural SIMT shape, with registers and ~2.8 KB of shared memory per warp (32+ warps per SM):
+// (836 warp instructions per point, issue-bound); a backward on the ring of view_attention_ring.cu halved the
+// instruction count but its 29 KB of shared memory per warp left 8 warps per SM (21 % issue-active,
+// latency-bound): 0.47 of the HBM peak.  Here a warp takes a GROUP of consecutive points holding at most 32
+// views and gives every kind of work its natural SIMT shape, with registers and ~2.8 KB of shared memory per
+// warp (32+ warps per SM):
 //   phase 1  LANE PER VIEW: scores, row id, the point's saved statistics -> attentions a, gate t (32 views
 //            per instruction; coalesced 16-byte score loads);
 //   phase 1b EVERY VIEW LANE issues ONE bulk async copy (cp.async.bulk -> UBLKCP) of its own row into the
@@ -25,40 +26,13 @@
 // A point with more than 32 views (never in the short-segment regime this kernel is dispatched for) is
 // walked in chunks of 32 views with its raw s' parked in grad_compat.
 // Requires G == 4 and the regular channel layout (a row is LPR = 4 * 2^k chunks of 16 bytes, <= 512 bytes).
-// HBM bytes per launch: those of the other two implementations (V (2 C s + 4 + 8 G) + N (C s + 8 + 12 G)).
+// HBM bytes per launch: those of the streaming backward (V (2 C s + 4 + 8 G) + N (C s + 8 + 12 G)).
 #include "view_attention.cuh"
 
 namespace dva {
 
 constexpr int kLaneWarps = 4;
 constexpr uint32_t kFull = 0xffffffffu;
-
-__device__ __forceinline__ uint32_t lane_smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void lane_mbar_init(uint32_t bar, uint32_t count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count) : "memory");
-}
-__device__ __forceinline__ void lane_mbar_expect_tx(uint32_t bar, uint32_t bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void lane_mbar_wait(uint32_t bar, uint32_t parity) {
-  uint32_t ok = 0;
-  while (!ok) {
-    asm volatile(
-        "{ .reg .pred p; mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2; selp.u32 %0, 1, 0, p; }"
-        : "=r"(ok) : "r"(bar), "r"(parity) : "memory");
-  }
-}
-__device__ __forceinline__ void lane_bulk_g2s(uint32_t dst, const void* src, uint32_t bytes, uint32_t bar) {
-  asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-               ::"r"(dst), "l"(src), "r"(bytes), "r"(bar) : "memory");
-}
-__device__ __forceinline__ void lane_fence_proxy_async() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
-
-__device__ __forceinline__ uint32_t lane_row_id(const void* idx, int idx64, int64_t v) {
-  if (idx == nullptr) return (uint32_t)v;
-  return idx64 ? (uint32_t) reinterpret_cast<const int64_t*>(idx)[v] : (uint32_t) reinterpret_cast<const int32_t*>(idx)[v];
-}
-__device__ __forceinline__ float pick4(const float4& v, int g) { return g == 0 ? v.x : (g == 1 ? v.y : (g == 2 ? v.z : v.w)); }
 
 struct LaneSmem {            // per warp
   float wt[32][4];           // a * t per (view, group)
@@ -83,11 +57,11 @@ va_lane_bwd_kernel(const VAParams P, const int PR) {
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   LaneSmem& sm = sm_all[warp];
   unsigned char* rows_s = rows_all + (size_t)warp * 32 * RS;
-  const uint32_t rows_u = lane_smem_u32(rows_s), bar_u = lane_smem_u32(&sm.bar);
+  const uint32_t rows_u = smem_u32(rows_s), bar_u = smem_u32(&sm.bar);
   uint32_t uses = 0;                                              // completed uses of the barrier (parity)
   if (lane == 0) {
-    lane_mbar_init(bar_u, 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    mbar_init(bar_u, 1);
+    fence_mbar_init();
   }
   __syncwarp();
   const int sg = lane / LPR, lir = lane % LPR, gk = lir / CPE;
@@ -106,14 +80,14 @@ va_lane_bwd_kernel(const VAParams P, const int PR) {
 
   // every view lane copies its own row into the warp's buffer; wait_rows() before the rows are read
   auto issue_rows = [&](int nv, uint32_t rid) {
-    lane_fence_proxy_async();                                     // earlier generic reads of the buffer come first
+    fence_proxy_async();                                     // earlier generic reads of the buffer come first
     __syncwarp();
-    if (lane == 0) lane_mbar_expect_tx(bar_u, (uint32_t)nv * row_bytes);
+    if (lane == 0) mbar_expect_tx(bar_u, (uint32_t)nv * row_bytes);
     __syncwarp();
-    if (lane < nv) lane_bulk_g2s(rows_u + (uint32_t)lane * RS, xbase + (uint64_t)rid * row_bytes, row_bytes, bar_u);
+    if (lane < nv) bulk_g2s(rows_u + (uint32_t)lane * RS, xbase + (uint64_t)rid * row_bytes, row_bytes, bar_u);
   };
   auto wait_rows = [&]() {
-    lane_mbar_wait(bar_u, uses & 1u);
+    mbar_wait(bar_u, uses & 1u);
     ++uses;
   };
 
@@ -193,7 +167,7 @@ va_lane_bwd_kernel(const VAParams P, const int PR) {
           const int64_t v = gvb + c0 + lane;
           float4 a = make_float4(0.f, 0.f, 0.f, 0.f);
           __syncwarp();
-          const uint32_t rid_l = lane < nv ? lane_row_id(P.idx, P.idx64, v) : 0u;
+          const uint32_t rid_l = lane < nv ? load_row_id(P.idx, P.idx64, v) : 0u;
           issue_rows(nv, rid_l);
           if (lane < nv) {
             const float4 c = __ldg(reinterpret_cast<const float4*>(P.compat) + v);
@@ -266,7 +240,7 @@ va_lane_bwd_kernel(const VAParams P, const int PR) {
       int4 sar = make_int4(-1, -1, -1, -1);
       const int64_t v = gvb + lane;
       __syncwarp();                                                 // previous group's tiles are free
-      const uint32_t rid_m = lane < nv ? lane_row_id(P.idx, P.idx64, v) : 0u;
+      const uint32_t rid_m = lane < nv ? load_row_id(P.idx, P.idx64, v) : 0u;
       if (nv > 0) issue_rows(nv, rid_m);                            // rows go in flight before anything else is loaded
       if (lane < nv) {
         const float4 c = __ldg(reinterpret_cast<const float4*>(P.compat) + v);

@@ -1,31 +1,27 @@
-// Ring implementation of the fused view-attention pair (same math and C ABI as view_attention.cu;
+// Ring forward of the fused view-attention pair (same math and C ABI as view_attention.cu;
 // reference chain: modules.py:518 row gather -> pooling.py:285-300 / 515-530).
 //
-// Why a second implementation.  ncu on the shipped-config shapes (S3DIS: 160 k points x ~8 views x
-// 64 ch) shows the streaming kernels ISSUE-bound, not HBM-bound: ~590 warp instructions per point,
-// of which only ~40 touch feature rows -- the rest is per-point scalar work (softmax statistics,
-// gating, pointer chasing) executed by a whole warp for one point at a time.  Here the two kinds
-// of work get the SIMT shape that suits them:
+// Why a second forward.  ncu on the shipped-config shapes (S3DIS: 160 k points x ~8 views x 64 ch)
+// shows the streaming kernels ISSUE-bound, not HBM-bound: ~590 warp instructions per point, of which
+// only ~40 touch feature rows -- the rest is per-point scalar work (softmax statistics, gating,
+// pointer chasing) executed by a whole warp for one point at a time.  Here the two kinds of work get
+// the SIMT shape that suits them:
 //
 //   * a warp owns a contiguous RANGE of points = a contiguous range of views, and streams that
 //     range's feature rows through a shared-memory ring as fixed-size BATCHES that ignore point
 //     boundaries: one 16-byte cp.async (LDGSTS) per lane and row step, S-1 batches in flight, row
 //     ids prefetched a batch ahead into one register per lane -- no load of the consumer sits on a
 //     dependent-address chain;
-//   * the consumer walks the range in GROUPS of up to 32 points (at most 256 / 128 views fwd / bwd):
+//   * the consumer walks the range in GROUPS of up to 32 points (at most 256 views):
 //       phase 1  LANE PER POINT: every lane computes the softmax statistics of its own point
 //                (max, first arg-max, denominator, gate) from the fp32 scores and leaves the final
 //                per-view weights e * t / den in a shared tile -- 32 points per instruction;
 //       phase 2  WARP PER ROW STEP: per point, weighted sum of its rows out of the ring
 //                (LDS.128 row chunk + LDS weight + VEC FFMA per row step), no arithmetic besides;
-//       phase 3  (backward) lane per point again: S = sum_v a s', grad_compat, gate gradients.
-//   * backward: the upstream-gradient rows of the next window of points are fetched by ONE elected
-//     lane with a bulk async copy (cp.async.bulk -> UBLKCP, completion on an mbarrier) -- they are
-//     contiguous in memory, the natural TMA case.
-//   * a point with more views than a group holds (never in the shipped configs) takes a warp-cooperative
-//     path: online softmax over the pieces of its segment (forward), raw s' parked in grad_compat
-//     (backward).
+//   * a point with more views than a group holds (never in the shipped configs) takes a
+//     warp-cooperative path: online softmax over the pieces of its segment.
 //
+// The backward of these shapes is the lane-per-view kernel (view_attention_lane.cu).
 // Requires G == 4 (every shipped config), rows of whole 16-byte chunks and at most 512 bytes;
 // everything else runs on the streaming kernels.  HBM bytes per launch are those of the streaming
 // kernels (see view_attention.cu).  exp is ex2.approx-based here (relative error ~1e-6).
@@ -39,20 +35,11 @@ namespace dva {
 #ifndef DVA_RING_WARPS
 #define DVA_RING_WARPS 1
 #endif
-#ifndef DVA_RING_PW_BYTES
-#define DVA_RING_PW_BYTES 4096    // backward: bytes of one grad_out window tile (x 2 buffers)
-#endif
 #ifndef DVA_RING_FWD_MINB
 #define DVA_RING_FWD_MINB 12      // CTAs per SM the register budget is sized for (x kRingWarps warps)
 #endif
-#ifndef DVA_RING_BWD_MINB
-#define DVA_RING_BWD_MINB 8
-#endif
 #ifndef DVA_RING_CAPV_FWD
 #define DVA_RING_CAPV_FWD 256     // views per point group (weight tile), multiple of 8
-#endif
-#ifndef DVA_RING_CAPV_BWD
-#define DVA_RING_CAPV_BWD 128
 #endif
 constexpr int kRingStages = DVA_RING_STAGES;
 constexpr int kRingWarps = DVA_RING_WARPS;     // warps of a CTA never synchronise with each other
@@ -63,66 +50,27 @@ constexpr uint32_t FULL = 0xffffffffu;
 #endif
 constexpr int kP1Unroll = DVA_RING_P1_UNROLL;   // score loads in flight per lane in the lane-per-point phases
 
-// Batch size (measured, tools/bench_shapes.py): forward likes 16 rows per batch for 128/256-byte
-// rows and more resident warps (2 KB batches) for 64- and 512-byte rows; backward 4 KB throughout.
-template <int LPR, bool BWD> struct RingGeom {
+// Batch size (measured, tools/bench_shapes.py): 16 rows per batch for 128/256-byte rows and more
+// resident warps (2 KB batches) for 64- and 512-byte rows.
+template <int LPR> struct RingGeom {
   static constexpr int RPI = 32 / LPR;                       // rows per warp step
   static constexpr int RS = LPR * 16;                        // row stride in the ring (bytes)
 #ifdef DVA_RING_BATCH_BYTES
   static constexpr int BATCH = DVA_RING_BATCH_BYTES;
 #else
-  static constexpr int BATCH = BWD ? 4096 : (LPR == 16 ? 4096 : 2048);
+  static constexpr int BATCH = LPR == 16 ? 4096 : 2048;
 #endif
   static constexpr int RB = (BATCH / RS) < 32 ? (BATCH / RS) : 32;   // rows per batch
   static constexpr int STEPS = RB / RPI;                     // row steps per batch
-  static constexpr int PW = (DVA_RING_PW_BYTES / RS) < 32 ? (DVA_RING_PW_BYTES / RS) : 32;   // points per window (bwd: grad_out tile rows)
-  static constexpr int MINB = BWD ? DVA_RING_BWD_MINB : (BATCH <= 2048 ? 16 : DVA_RING_FWD_MINB);
+  static constexpr int MINB = BATCH <= 2048 ? 16 : DVA_RING_FWD_MINB;
   static_assert(RB >= RPI && RB % RPI == 0 && (RB & (RB - 1)) == 0, "batch geometry");
 };
 
-__device__ __forceinline__ uint32_t smem_u32(const void* p) {
-  return (uint32_t)__cvta_generic_to_shared(p);
-}
-__device__ __forceinline__ void cp_async16(uint32_t dst, const void* src) {
-  asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(dst), "l"(src) : "memory");
-}
-__device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
-template <int N> __device__ __forceinline__ void cp_async_wait() {
-  asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory");
-}
-// ---- mbarrier + bulk async copy (backward: contiguous grad_out rows of a window of points)
-__device__ __forceinline__ void mbar_init(uint32_t bar, uint32_t count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count) : "memory");
-}
-__device__ __forceinline__ void mbar_expect_tx(uint32_t bar, uint32_t bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
-  uint32_t ok = 0;
-  while (!ok) {
-    asm volatile(
-        "{ .reg .pred p; mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2; selp.u32 %0, 1, 0, p; }"
-        : "=r"(ok) : "r"(bar), "r"(parity) : "memory");
-  }
-}
-__device__ __forceinline__ void bulk_g2s(uint32_t dst, const void* src, uint32_t bytes, uint32_t bar) {
-  asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-               ::"r"(dst), "l"(src), "r"(bytes), "r"(bar) : "memory");
-}
-__device__ __forceinline__ void fence_proxy_async() {
-  asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-}
 __device__ __forceinline__ void prefetch_l2(const void* p) {
   asm volatile("prefetch.global.L2 [%0];" ::"l"(p));
 }
 
-__device__ __forceinline__ uint32_t load_row_id(const void* idx, int idx64, int64_t v) {
-  if (idx == nullptr) return (uint32_t)v;
-  return idx64 ? (uint32_t) reinterpret_cast<const int64_t*>(idx)[v]
-               : (uint32_t) reinterpret_cast<const int32_t*>(idx)[v];
-}
-
-// weight / attention tiles hold one float4 (4 groups) per view, 8 views per 36-float row: lanes
+// the weight tile holds one float4 (4 groups) per view, 8 views per 36-float row: lanes
 // that walk their own points at a stride of 8k views still hit distinct banks
 __device__ __forceinline__ int tix(int u) { return (u + (u >> 3)) << 2; }
 constexpr int tile_floats(int capv) { return (capv / 8) * 36; }
@@ -131,46 +79,38 @@ __device__ __forceinline__ float sel4(const float4& v, int g) {
   return g == 0 ? v.x : (g == 1 ? v.y : (g == 2 ? v.z : v.w));
 }
 
-// per-warp shared memory (bytes)
-template <int LPR, bool BWD> struct RingSmem {
-  using Gm = RingGeom<LPR, BWD>;
-  size_t rows, tile, tile2, rowid, gout, tpt, bars, total;
+// per-warp shared memory (bytes): the ring, the weight tile, the output scale per point of the group
+template <int LPR> struct RingSmem {
+  using Gm = RingGeom<LPR>;
+  size_t rows, tile, tpt, total;
   __host__ __device__ RingSmem() {
-    constexpr bool bwd = BWD;
     rows = (size_t)kRingStages * Gm::RB * Gm::RS;
-    tile = (size_t)tile_floats(bwd ? DVA_RING_CAPV_BWD : DVA_RING_CAPV_FWD) * sizeof(float);
-    tile2 = bwd ? tile : 0;
-    rowid = bwd ? (size_t)kRingStages * Gm::RB * sizeof(uint32_t) : 0;
-    gout = bwd ? (size_t)2 * Gm::PW * Gm::RS : 0;
-    tpt = (size_t)32 * kRG * sizeof(float);    // per-point scale (fwd) / gate (bwd) of the group
-    bars = bwd ? 16 : 0;
-    total = rows + tile + tile2 + rowid + gout + tpt + bars;
+    tile = (size_t)tile_floats(DVA_RING_CAPV_FWD) * sizeof(float);
+    tpt = (size_t)32 * kRG * sizeof(float);
+    total = rows + tile + tpt;
   }
 };
 
-// window of points [pg, pg + W): lane k < W holds the range-relative first view and the view
-// count of point pg + k (0 views past the end of the range)
+// window of points [pg, pg + 32): lane k holds the range-relative first view and the view count
+// of point pg + k (0 views past the end of the range)
 __device__ __forceinline__ void load_window(const int64_t* __restrict__ ptr, int64_t pg, int64_t pb,
-                                            int64_t vb, int lane, int W, int& pl, int& cnt) {
+                                            int64_t vb, int lane, int& pl, int& cnt) {
   const int64_t q0 = (pg + lane < pb) ? pg + lane : pb;
   const int64_t q1 = (q0 + 1 < pb) ? q0 + 1 : pb;
   pl = (int)(ptr[q0] - vb);
-  cnt = (lane < W) ? (int)(ptr[q1] - vb) - pl : 0;
+  cnt = (int)(ptr[q1] - vb) - pl;
 }
 
-// ---------------------------------------------------------------------------------------------
-// forward
-// ---------------------------------------------------------------------------------------------
 template <typename T, int LPR>
-__global__ void __launch_bounds__(kRingWarps * 32, RingGeom<LPR, false>::MINB)
+__global__ void __launch_bounds__(kRingWarps * 32, RingGeom<LPR>::MINB)
 va_ring_fwd_kernel(const VAParams P, const int PR) {
-  using Gm = RingGeom<LPR, false>;
+  using Gm = RingGeom<LPR>;
   constexpr int VEC = Vec16<T>::N, RPI = Gm::RPI, RB = Gm::RB, RS = Gm::RS, S = kRingStages;
   constexpr int G = kRG, CAPV = DVA_RING_CAPV_FWD;
   extern __shared__ __align__(128) unsigned char smem_raw[];
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int C = P.C;
-  const RingSmem<LPR, false> L;
+  const RingSmem<LPR> L;
   unsigned char* base = smem_raw + (size_t)warp * L.total;
   unsigned char* rows_s = base;
   float* wt = reinterpret_cast<float*>(base + L.rows);
@@ -261,7 +201,7 @@ va_ring_fwd_kernel(const VAParams P, const int PR) {
     for (int bi = 0; bi < S - 1; ++bi) issue(bi);
     int cb = -1;                                    // newest batch known to be resident
     int pl, cnt;
-    load_window(P.ptr, pa, pb, vb, lane, 32, pl, cnt);
+    load_window(P.ptr, pa, pb, vb, lane, pl, cnt);
 
     for (int64_t pg = pa; pg < pb;) {
       // group = longest prefix of the window with at most CAPV views
@@ -276,7 +216,7 @@ va_ring_fwd_kernel(const VAParams P, const int PR) {
         const int s = gs0;
         const int64_t i = pg;
         int pl_n, cnt_n;
-        load_window(P.ptr, pg + 1, pb, vb, lane, 32, pl_n, cnt_n);
+        load_window(P.ptr, pg + 1, pb, vb, lane, pl_n, cnt_n);
         const float inv_sq = P.group_scaling ? rsqrtf((float)n) : 1.f;
         const int gl = lane & (G - 1);
         const float* __restrict__ cp = P.compat + (vb + s) * G;
@@ -339,7 +279,7 @@ va_ring_fwd_kernel(const VAParams P, const int PR) {
 
       int pl_n = 0, cnt_n = 0;                      // next window: loaded a group early
       if (pg + kmax < pb) {
-        load_window(P.ptr, pg + kmax, pb, vb, lane, 32, pl_n, cnt_n);
+        load_window(P.ptr, pg + kmax, pb, vb, lane, pl_n, cnt_n);
         // warm the next group's scores in L2: 32 lanes x 128 bytes = the next 256 views
         const int64_t pv = vb + __shfl_sync(FULL, pl + cnt, kmax - 1) + lane * 8;
         if (pv < P.V) prefetch_l2(P.compat + pv * G);
@@ -439,381 +379,6 @@ va_ring_fwd_kernel(const VAParams P, const int PR) {
 }
 
 // ---------------------------------------------------------------------------------------------
-// backward (math: see view_attention.cu; regular group layout only)
-// ---------------------------------------------------------------------------------------------
-template <typename T, int LPR>
-__global__ void __launch_bounds__(kRingWarps * 32, RingGeom<LPR, true>::MINB)
-va_ring_bwd_kernel(const VAParams P, const int PR) {
-  using Gm = RingGeom<LPR, true>;
-  constexpr int VEC = Vec16<T>::N, RPI = Gm::RPI, RB = Gm::RB, RS = Gm::RS, S = kRingStages;
-  constexpr int G = kRG, CAPV = DVA_RING_CAPV_BWD, PW = Gm::PW;
-  extern __shared__ __align__(128) unsigned char smem_raw[];
-  __shared__ float gate_s[kRingWarps][2 * kRG];
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int C = P.C;
-  const RingSmem<LPR, true> L;
-  unsigned char* base = smem_raw + (size_t)warp * L.total;
-  unsigned char* rows_s = base;
-  float* at = reinterpret_cast<float*>(base + L.rows);                // attentions a_vg
-  float* st = reinterpret_cast<float*>(base + L.rows + L.tile);       // s'_vg
-  uint32_t* rowid_s = reinterpret_cast<uint32_t*>(base + L.rows + L.tile + L.tile2);
-  unsigned char* gout_s = base + L.rows + L.tile + L.tile2 + L.rowid;
-  float* tpt = reinterpret_cast<float*>(gout_s + L.gout);             // gate t per point of the group
-  uint64_t* bars = reinterpret_cast<uint64_t*>(gout_s + L.gout + L.tpt);
-  const uint32_t rows_u = smem_u32(rows_s), gout_u = smem_u32(gout_s);
-  const uint32_t bar_u[2] = {smem_u32(bars), smem_u32(bars + 1)};
-
-  for (int q = lane; q < (int)(L.rows / 16); q += 32) reinterpret_cast<uint4*>(rows_s)[q] = make_uint4(0u, 0u, 0u, 0u);
-  for (int q = lane; q < (int)(L.gout / 16); q += 32) reinterpret_cast<uint4*>(gout_s)[q] = make_uint4(0u, 0u, 0u, 0u);
-  if (lane == 0) {
-    mbar_init(bar_u[0], 1);
-    mbar_init(bar_u[1], 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-  }
-  fence_proxy_async();
-  __syncwarp();
-
-  const int sg = lane / LPR, lir = lane % LPR;
-  const bool live = lir * VEC < C;
-  const int gk = group_of_channel(live ? lir * VEC : 0, C, G);
-  const uint32_t row_bytes = (uint32_t)C * sizeof(T);
-  const char* __restrict__ xb = reinterpret_cast<const char*>(P.x) + (live ? lir * 16 : 0);
-  char* __restrict__ gxb = reinterpret_cast<char*>(P.gx) + (live ? lir * 16 : 0);
-  const bool gating = P.gate_w != nullptr;
-  float4 gw4 = make_float4(0.f, 0.f, 0.f, 0.f), gb4 = gw4;
-  if (gating) {
-    gw4 = make_float4(P.gate_w[0], P.gate_w[1], P.gate_w[2], P.gate_w[3]);
-    gb4 = make_float4(P.gate_b[0], P.gate_b[1], P.gate_b[2], P.gate_b[3]);
-  }
-  float4 dw4 = make_float4(0.f, 0.f, 0.f, 0.f), db4 = dw4;          // gate gradients (lane partials)
-  const bool has_idx = P.idx != nullptr;
-  const bool scatter = P.scatter && has_idx;
-  const bool padded = row_bytes != (uint32_t)RS;    // rows narrower than the ring stride: per-row tile copies
-  // regular layout with G = 4 and a power-of-two chunk count (host): a row is exactly LPR chunks,
-  // the lanes that share a group form aligned blocks of CPE = LPR / 4 lanes
-  constexpr int CPE = LPR / kRG;
-  const bool leader = (lir & (CPE - 1)) == 0;
-  uint32_t uses0 = 0, uses1 = 0;                    // completed uses of grad_out buffer 0 / 1 (mbarrier parity)
-
-  const int64_t n_ranges = (P.N + PR - 1) / PR;
-  const int64_t warps_total = (int64_t)gridDim.x * kRingWarps;
-  for (int64_t r = (int64_t)blockIdx.x * kRingWarps + warp; r < n_ranges; r += warps_total) {
-    const int64_t pa = r * PR;
-    const int64_t pb = (pa + PR < P.N) ? pa + PR : P.N;
-    const int64_t vb = P.ptr[pa];
-    const int nv = (int)(P.ptr[pb] - vb);
-    uint32_t rid = (lane < RB && lane < nv) ? load_row_id(P.idx, P.idx64, vb + lane) : 0u;
-
-    auto issue = [&](int bi) {
-      const int slot = bi % S;
-      const int v0 = bi * RB;
-      const int nrows = (nv - v0 < RB) ? nv - v0 : RB;
-      if (nrows > 0) {
-        const uint32_t dst0 = rows_u + (uint32_t)(slot * RB) * RS + lir * 16;
-#pragma unroll
-        for (int stp = 0; stp < Gm::STEPS; ++stp) {
-          const int rr = stp * RPI + sg;
-          const uint32_t srow = __shfl_sync(FULL, rid, rr);
-          if (rr < nrows && live) cp_async16(dst0 + rr * RS, xb + (uint64_t)srow * row_bytes);
-        }
-        if (lane < nrows) rowid_s[slot * RB + lane] = scatter ? rid : (uint32_t)(vb + v0 + lane);   // dx row
-      }
-      cp_async_commit();
-      const int v1 = v0 + RB;
-      rid = (lane < RB && v1 + lane < nv) ? load_row_id(P.idx, P.idx64, vb + v1 + lane) : 0u;
-    };
-    auto advance_to = [&](int b, int& cb) {
-      while (cb < b) {
-        __syncwarp();
-        ++cb;
-        issue(cb + S - 1);
-        cp_async_wait<S - 1>();
-        __syncwarp();
-      }
-    };
-    // grad_out rows of the window [p0, p0 + PW) -> buffer j, one mbarrier phase
-    auto fetch_window = [&](int64_t p0, int j) {
-      const int np = (pb - p0 < PW) ? (int)(pb - p0) : PW;
-      if (lane == 0) {
-        fence_proxy_async();                        // earlier generic reads of this buffer come first
-        mbar_expect_tx(bar_u[j], (uint32_t)np * row_bytes);
-        const char* gsrc = reinterpret_cast<const char*>(P.gout) + p0 * (int64_t)row_bytes;
-        const uint32_t gdst = gout_u + (uint32_t)(j * PW) * RS;
-        if (!padded) {
-          bulk_g2s(gdst, gsrc, (uint32_t)np * row_bytes, bar_u[j]);
-        } else {
-          for (int q = 0; q < np; ++q) bulk_g2s(gdst + q * RS, gsrc + (size_t)q * row_bytes, row_bytes, bar_u[j]);
-        }
-      }
-    };
-    // rows of one piece: dx = a * gd (stored), s' = <gd, x> per (view, group) -> s tile
-    auto piece_rows = [&](int slot, int lo, int np, int u0, const float (&gd)[VEC]) {
-      const unsigned char* rp = rows_s + (size_t)(slot * RB + lo) * RS + lir * 16;
-      const uint32_t* op = rowid_s + slot * RB + lo;
-#pragma unroll 4
-      for (int v0 = sg; v0 < np + sg; v0 += RPI) {  // warp-uniform trip count
-        const bool ok = v0 < np;
-        const int vv = ok ? v0 : 0;
-        const uint4 raw = *reinterpret_cast<const uint4*>(rp + (size_t)vv * RS);
-        const int ti = tix(u0 + vv) + gk;
-        const float a = at[ti];
-        const uint32_t orow = op[vv];
-        float fv[VEC], dx[VEC];
-        unpack16<T, VEC>(raw, fv);
-        float dot = 0.f;
-#pragma unroll
-        for (int j = 0; j < VEC; ++j) {
-          dot = fmaf(gd[j], fv[j], dot);
-          dx[j] = a * gd[j];
-        }
-        if (ok && live) stg_stream16(gxb + (uint64_t)orow * row_bytes, pack16<T, VEC>(dx));
-        float rsum = dot;
-#pragma unroll
-        for (int o = 1; o < CPE; o <<= 1) rsum += __shfl_xor_sync(FULL, rsum, o);
-        if (ok && leader) st[ti] = rsum;
-      }
-    };
-
-#pragma unroll
-    for (int bi = 0; bi < S - 1; ++bi) issue(bi);
-    int cb = -1;
-    __syncwarp();
-    fetch_window(pa, 0);
-    int jbuf = 0;
-    int pl, cnt;
-    load_window(P.ptr, pa, pb, vb, lane, PW, pl, cnt);
-    float4 smx, sdn; int4 sar;                       // saved statistics of point pg + lane
-    {
-      const int64_t q = (pa + lane < pb) ? pa + lane : pa;
-      smx = reinterpret_cast<const float4*>(P.s_max)[q];
-      sdn = reinterpret_cast<const float4*>(P.s_den)[q];
-      sar = reinterpret_cast<const int4*>(P.s_arg)[q];
-    }
-
-    for (int64_t pg = pa; pg < pb; jbuf ^= 1) {
-      const int gs0 = __shfl_sync(FULL, pl, 0);
-      const bool fits = (lane < PW) && (pg + lane < pb) && (pl + cnt - gs0 <= CAPV);
-      const unsigned fm = __ballot_sync(FULL, fits);
-      const int kfit = (fm == FULL) ? 32 : __ffs(~fm) - 1;
-      const int kmax = kfit > 0 ? kfit : 1;         // a point too long for the tile is a group of its own
-      const bool longpt = kfit == 0;
-
-      // next window: pointers, statistics and (bulk copy) grad_out rows go in flight now
-      int pl_n = 0, cnt_n = 0;
-      float4 smx_n = smx, sdn_n = sdn; int4 sar_n = sar;
-      __syncwarp();                                 // every lane is done with the other grad_out buffer
-      if (pg + kmax < pb) {
-        const int64_t p1 = pg + kmax;
-        load_window(P.ptr, p1, pb, vb, lane, PW, pl_n, cnt_n);
-        const int64_t q = (p1 + lane < pb) ? p1 + lane : p1;
-        smx_n = reinterpret_cast<const float4*>(P.s_max)[q];
-        sdn_n = reinterpret_cast<const float4*>(P.s_den)[q];
-        sar_n = reinterpret_cast<const int4*>(P.s_arg)[q];
-        fetch_window(p1, jbuf ^ 1);
-        const int64_t pv = vb + __shfl_sync(FULL, pl + cnt, kmax - 1) + lane * 8;
-        if (pv < P.V) prefetch_l2(P.compat + pv * G);
-      }
-      {
-        const uint32_t par = (jbuf ? uses1 : uses0) & 1u;
-        mbar_wait(bar_u[jbuf], par);
-        if (jbuf) ++uses1; else ++uses0;
-      }
-      const unsigned char* gtile = gout_s + (size_t)(jbuf * PW) * RS + lir * 16;
-
-      if (longpt) {
-        // ---- one point with more views than the tiles hold: warp-cooperative, raw s' parked in grad_compat
-        const int n = __shfl_sync(FULL, cnt, 0);
-        const int s = gs0;
-        const int gl = lane & (G - 1);
-        const float m = sel4(make_float4(__shfl_sync(FULL, smx.x, 0), __shfl_sync(FULL, smx.y, 0),
-                                         __shfl_sync(FULL, smx.z, 0), __shfl_sync(FULL, smx.w, 0)), gl);
-        const float dnv = sel4(make_float4(__shfl_sync(FULL, sdn.x, 0), __shfl_sync(FULL, sdn.y, 0),
-                                           __shfl_sync(FULL, sdn.z, 0), __shfl_sync(FULL, sdn.w, 0)), gl);
-        const int a0 = __shfl_sync(FULL, sar.x, 0), a1 = __shfl_sync(FULL, sar.y, 0);
-        const int a2 = __shfl_sync(FULL, sar.z, 0), a3 = __shfl_sync(FULL, sar.w, 0);
-        const int arg_v = gl == 0 ? a0 : (gl == 1 ? a1 : (gl == 2 ? a2 : a3));
-        const float inv_den = 1.f / dnv;
-        const float inv_sq = P.group_scaling ? rsqrtf((float)n) : 1.f;
-        const float gwl = sel4(gw4, gl), gbl = sel4(gb4, gl);
-        const float z = fmaf(gwl, m, gbl);
-        const float t = gating ? tanhf(fmaxf(z, 0.f)) : 1.f;
-        float gd[VEC];
-        {
-          const uint4 raw = *reinterpret_cast<const uint4*>(gtile);
-          unpack16<T, VEC>(raw, gd);
-          const float tk = __shfl_sync(FULL, t, gk);
-#pragma unroll
-          for (int j = 0; j < VEC; ++j) gd[j] = live ? gd[j] * tk : 0.f;
-        }
-        const float* __restrict__ cp = P.compat + (vb + s) * G;
-        float* gc = P.gcompat + (vb + s) * G;
-        float Ssum = 0.f;
-        const int vend = s + n;
-        for (int v = s; v < vend;) {
-          const int b = v / RB, lo = v % RB;
-          const int np = (RB - lo < vend - v) ? RB - lo : vend - v;
-          advance_to(b, cb);
-          const int npG = np * G;
-          __syncwarp();
-          for (int e = lane; e < npG; e += 32)
-            at[tix(e / G) + gl] = __expf((__ldg(cp + (size_t)(v - s) * G + e) - m) * inv_sq) * inv_den;
-          __syncwarp();
-          piece_rows(b % S, lo, np, 0, gd);
-          __syncwarp();
-          for (int e = lane; e < npG; e += 32) {
-            const int ti = tix(e / G) + gl;
-            const float sv = st[ti];
-            Ssum = fmaf(at[ti], sv, Ssum);
-            gc[(size_t)(v - s) * G + e] = sv;       // raw s': finalised below once S is complete
-          }
-          v += np;
-        }
-        Ssum = group_lane_sum(Ssum, G);
-        const float one_m_t2 = 1.f - t * t;
-        const float dLdt = (t != 0.f) ? Ssum / t : 0.f;
-        const bool open = gating && z > 0.f;
-        const float dq = open ? dLdt * one_m_t2 * gwl : 0.f;
-        if (open && lane < G) {
-          const float dwv = dLdt * one_m_t2 * m, dbv = dLdt * one_m_t2;
-          if (lane == 0) { dw4.x += dwv; db4.x += dbv; }
-          if (lane == 1) { dw4.y += dwv; db4.y += dbv; }
-          if (lane == 2) { dw4.z += dwv; db4.z += dbv; }
-          if (lane == 3) { dw4.w += dwv; db4.w += dbv; }
-        }
-        __syncwarp();                               // raw s' written by other lanes of this warp
-        const int first_view = (int)(vb + s);
-        for (int e = lane; e < n * G; e += 32) {
-          const float a = __expf((__ldg(cp + e) - m) * inv_sq) * inv_den;
-          float d = a * (__ldcg(gc + e) - Ssum) * inv_sq;
-          if (first_view + e / G == arg_v) d += dq;
-          gc[e] = d;
-        }
-        __syncwarp();
-        pg += 1; pl = pl_n; cnt = cnt_n; smx = smx_n; sdn = sdn_n; sar = sar_n;
-        continue;
-      }
-
-      // ---- phase 1: lane k owns point pg + k: attentions a_vg -> tile, gate t -> tpt
-      const float inv_sq_l = (P.group_scaling && cnt > 0) ? rsqrtf((float)cnt) : 1.f;
-      float4 t4 = make_float4(1.f, 1.f, 1.f, 1.f), z4 = t4;
-      if (lane < kmax && cnt > 0) {
-        const float4* __restrict__ cp = reinterpret_cast<const float4*>(P.compat + (vb + pl) * G);
-        const int u0 = pl - gs0;
-        const float4 id = make_float4(1.f / sdn.x, 1.f / sdn.y, 1.f / sdn.z, 1.f / sdn.w);
-        for (int j0 = 0; j0 < cnt; j0 += kP1Unroll) {
-          float4 c[kP1Unroll];
-#pragma unroll
-          for (int u = 0; u < kP1Unroll; ++u)
-            c[u] = (j0 + u < cnt) ? __ldg(cp + j0 + u) : make_float4(0.f, 0.f, 0.f, 0.f);
-#pragma unroll
-          for (int u = 0; u < kP1Unroll; ++u) {
-            if (j0 + u < cnt) {
-              float4 a;
-              a.x = __expf((c[u].x - smx.x) * inv_sq_l) * id.x; a.y = __expf((c[u].y - smx.y) * inv_sq_l) * id.y;
-              a.z = __expf((c[u].z - smx.z) * inv_sq_l) * id.z; a.w = __expf((c[u].w - smx.w) * inv_sq_l) * id.w;
-              *reinterpret_cast<float4*>(at + tix(u0 + j0 + u)) = a;
-            }
-          }
-        }
-        if (gating) {
-          z4 = make_float4(fmaf(gw4.x, smx.x, gb4.x), fmaf(gw4.y, smx.y, gb4.y),
-                           fmaf(gw4.z, smx.z, gb4.z), fmaf(gw4.w, smx.w, gb4.w));
-          t4 = make_float4(tanhf(fmaxf(z4.x, 0.f)), tanhf(fmaxf(z4.y, 0.f)),
-                           tanhf(fmaxf(z4.z, 0.f)), tanhf(fmaxf(z4.w, 0.f)));
-        }
-      }
-      reinterpret_cast<float4*>(tpt)[lane] = t4;
-      __syncwarp();
-
-      // ---- phase 2: per point, rows out of the ring: dx stores + s' tile
-      for (int k = 0; k < kmax; ++k) {
-        const int s = __shfl_sync(FULL, pl, k);
-        const int n = __shfl_sync(FULL, cnt, k);
-        if (n == 0) continue;                       // no view: nothing flows back
-        float gd[VEC];
-        {
-          const uint4 raw = *reinterpret_cast<const uint4*>(gtile + (size_t)k * RS);
-          unpack16<T, VEC>(raw, gd);
-          const float tk = tpt[k * G + gk];
-#pragma unroll
-          for (int j = 0; j < VEC; ++j) gd[j] = live ? gd[j] * tk : 0.f;
-        }
-        const int vend = s + n;
-        for (int v = s; v < vend;) {
-          const int b = v / RB, lo = v % RB;
-          const int np = (RB - lo < vend - v) ? RB - lo : vend - v;
-          advance_to(b, cb);
-          piece_rows(b % S, lo, np, v - gs0, gd);
-          v += np;
-        }
-      }
-      __syncwarp();
-
-      // ---- phase 3: lane k: S = sum_v a s', grad_compat, gate gradients
-      if (lane < kmax && cnt > 0) {
-        const int u0 = pl - gs0;
-        float4 Ss = make_float4(0.f, 0.f, 0.f, 0.f);
-        for (int j = 0; j < cnt; ++j) {
-          const float4 a = *reinterpret_cast<const float4*>(at + tix(u0 + j));
-          const float4 sv = *reinterpret_cast<const float4*>(st + tix(u0 + j));
-          Ss.x = fmaf(a.x, sv.x, Ss.x); Ss.y = fmaf(a.y, sv.y, Ss.y);
-          Ss.z = fmaf(a.z, sv.z, Ss.z); Ss.w = fmaf(a.w, sv.w, Ss.w);
-        }
-        float4 dq = make_float4(0.f, 0.f, 0.f, 0.f);
-        if (gating) {
-#define DVA_GATE_TERM(c)                                                                  \
-          if (z4.c > 0.f) {                                                               \
-            const float dLdt = (t4.c != 0.f) ? Ss.c / t4.c : 0.f;                         \
-            const float u = dLdt * (1.f - t4.c * t4.c);                                   \
-            dq.c = u * gw4.c; dw4.c += u * smx.c; db4.c += u;                             \
-          }
-          DVA_GATE_TERM(x) DVA_GATE_TERM(y) DVA_GATE_TERM(z) DVA_GATE_TERM(w)
-#undef DVA_GATE_TERM
-        }
-        float4* __restrict__ gc = reinterpret_cast<float4*>(P.gcompat + (vb + pl) * G);
-        const int fv0 = (int)(vb + pl);
-        for (int j = 0; j < cnt; ++j) {
-          const float4 a = *reinterpret_cast<const float4*>(at + tix(u0 + j));
-          const float4 sv = *reinterpret_cast<const float4*>(st + tix(u0 + j));
-          float4 d;
-          d.x = a.x * (sv.x - Ss.x) * inv_sq_l; d.y = a.y * (sv.y - Ss.y) * inv_sq_l;
-          d.z = a.z * (sv.z - Ss.z) * inv_sq_l; d.w = a.w * (sv.w - Ss.w) * inv_sq_l;
-          if (fv0 + j == sar.x) d.x += dq.x;
-          if (fv0 + j == sar.y) d.y += dq.y;
-          if (fv0 + j == sar.z) d.z += dq.z;
-          if (fv0 + j == sar.w) d.w += dq.w;
-          gc[j] = d;
-        }
-      }
-      __syncwarp();                                 // tiles are rewritten by the next group
-      pg += kmax; pl = pl_n; cnt = cnt_n; smx = smx_n; sdn = sdn_n; sar = sar_n;
-    }
-    cp_async_wait<0>();
-    __syncwarp();
-  }
-
-  // ---- gate parameter gradients: lanes -> warp -> block partial (fixed order), block -> workspace
-  if (P.gate_partial != nullptr) {
-    float v[8] = {dw4.x, dw4.y, dw4.z, dw4.w, db4.x, db4.y, db4.z, db4.w};
-#pragma unroll
-    for (int q = 0; q < 8; ++q) {
-#pragma unroll
-      for (int o = 16; o > 0; o >>= 1) v[q] += __shfl_xor_sync(FULL, v[q], o);
-    }
-    if (lane == 0) {
-#pragma unroll
-      for (int q = 0; q < 8; ++q) gate_s[warp][q] = v[q];
-    }
-    __syncthreads();
-    if ((int)threadIdx.x < 2 * G) {
-      float acc = 0.f;
-      for (int w = 0; w < kRingWarps; ++w) acc += gate_s[w][threadIdx.x];
-      P.gate_partial[(int64_t)blockIdx.x * 2 * G + threadIdx.x] = acc;
-    }
-  }
-}
-
-// ---------------------------------------------------------------------------------------------
 // host side
 // ---------------------------------------------------------------------------------------------
 template <typename T> static int ring_lpr(const VAParams& P) {
@@ -824,36 +389,19 @@ template <typename T> static int ring_lpr(const VAParams& P) {
   return 32;
 }
 
-template <typename T>
-static bool ring_common_ok(const VAParams& P, const void* o1, const void* o2) {
+template <typename T> static bool ring_fwd_ok(const VAParams& P) {
   constexpr int V16 = Vec16<T>::N;
   const int C = P.C, G = P.G;
   if (G != kRG) return false;
   if (C % V16 != 0 || C / V16 > 32) return false;   // rows of at most 512 bytes, whole 16-byte chunks
-  if (!aligned16(P.x) || !aligned16(o1) || (o2 != nullptr && !aligned16(o2))) return false;
-  if (!aligned16(P.compat)) return false;
+  if (!aligned16(P.x) || !aligned16(P.out) || !aligned16(P.compat)) return false;
+  if (P.att != nullptr && !aligned16(P.att)) return false;
+  if (P.seg_max != nullptr && (!aligned16(P.seg_max) || !aligned16(P.seg_den) || !aligned16(P.seg_arg))) return false;
   if (P.V >= (1ll << 31) || P.R >= (1ll << 32)) return false;
   for (int c0 = 0; c0 < C; c0 += V16)               // chunks never straddle channel groups
     if (group_of_channel(c0, C, G) != group_of_channel(c0 + V16 - 1, C, G)) return false;
   return true;
 }
-
-template <typename T> static bool ring_fwd_ok(const VAParams& P) {
-  if (!ring_common_ok<T>(P, P.out, nullptr)) return false;
-  if (P.att != nullptr && !aligned16(P.att)) return false;
-  if (P.seg_max != nullptr && (!aligned16(P.seg_max) || !aligned16(P.seg_den) || !aligned16(P.seg_arg))) return false;
-  return true;
-}
-template <typename T> static bool ring_bwd_ok(const VAParams& P) {
-  constexpr int V16 = Vec16<T>::N;
-  if (!ring_common_ok<T>(P, P.gout, P.gx)) return false;
-  if (P.C % P.G != 0 || (P.C / P.G) % V16 != 0) return false;
-  const int cpg = (P.C / P.G) / V16;
-  if ((cpg & (cpg - 1)) != 0) return false;         // regular layout: a row is 4 * cpg = LPR chunks
-  if (!aligned16(P.s_max) || !aligned16(P.s_den) || !aligned16(P.s_arg) || !aligned16(P.gcompat)) return false;
-  return true;
-}
-
 bool va_ring_fwd_applicable(const VAParams& P, int dtype) {
   switch (dtype) {
     case DVA_F32: return ring_fwd_ok<float>(P);
@@ -862,58 +410,30 @@ bool va_ring_fwd_applicable(const VAParams& P, int dtype) {
     default: return false;
   }
 }
-bool va_ring_bwd_applicable(const VAParams& P, int dtype) {
-  switch (dtype) {
-    case DVA_F32: return ring_bwd_ok<float>(P);
-    case DVA_BF16: return ring_bwd_ok<__nv_bfloat16>(P);
-    case DVA_F16: return ring_bwd_ok<__half>(P);
-    default: return false;
-  }
-}
 
 // grid = co-resident CTAs (148 SMs x occupancy); PR = points per range (one range per warp when
 // the problem is large enough, never fewer than 8 points)
-template <typename K>
-static int ring_launch_geometry(K kern, size_t smem, int64_t N, int max_ctas_per_sm, int* grid_out, int* pr_out) {
+template <typename T, int LPR>
+static int ring_fwd_launch(const VAParams& P, cudaStream_t st) {
+  const RingSmem<LPR> L;
+  const size_t smem = L.total * kRingWarps;
+  auto kern = va_ring_fwd_kernel<T, LPR>;
   cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   if (e != cudaSuccess) return failf((int)e, "view_attention ring: %zu bytes of shared memory: %s", smem, cudaGetErrorString(e));
   int occ = 0;
   if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, kRingWarps * 32, smem) != cudaSuccess || occ < 1) occ = 1;
-  if (occ > max_ctas_per_sm) occ = max_ctas_per_sm;
+  if (occ > 32) occ = 32;
   int64_t grid = (int64_t)kNumSMs * occ;
   const int64_t warps = grid * kRingWarps;
-  int64_t pr = (N + warps - 1) / warps;
+  int64_t pr = (P.N + warps - 1) / warps;
   if (pr < 8) pr = 8;
-  const int64_t n_ranges = (N + pr - 1) / pr;
+  const int64_t n_ranges = (P.N + pr - 1) / pr;
   const int64_t need = (n_ranges + kRingWarps - 1) / kRingWarps;
   if (grid > need) grid = need;
   if (grid < 1) grid = 1;
-  *grid_out = (int)grid; *pr_out = (int)pr;
-  return DVA_OK;
-}
-
-template <typename T, int LPR>
-static int ring_fwd_launch(const VAParams& P, cudaStream_t st) {
-  const RingSmem<LPR, false> L;
-  const size_t smem = L.total * kRingWarps;
-  auto kern = va_ring_fwd_kernel<T, LPR>;
-  int grid, pr;
-  if (int rc = ring_launch_geometry(kern, smem, P.N, 32, &grid, &pr)) return rc;
-  kern<<<grid, kRingWarps * 32, smem, st>>>(P, pr);
+  kern<<<(int)grid, kRingWarps * 32, smem, st>>>(P, (int)pr);
   return check_launch("view_attention_fwd(ring)");
 }
-template <typename T, int LPR>
-static int ring_bwd_launch(const VAParams& P, int* grid_out, cudaStream_t st) {
-  const RingSmem<LPR, true> L;
-  const size_t smem = L.total * kRingWarps;
-  auto kern = va_ring_bwd_kernel<T, LPR>;
-  int grid, pr;
-  if (int rc = ring_launch_geometry(kern, smem, P.N, 8, &grid, &pr)) return rc;   // gate-gradient workspace: 148 x 8 partials
-  *grid_out = grid;
-  kern<<<grid, kRingWarps * 32, smem, st>>>(P, pr);
-  return check_launch("view_attention_bwd(ring)");
-}
-
 template <typename T> static int ring_fwd_typed(const VAParams& P, cudaStream_t st) {
   switch (ring_lpr<T>(P)) {
     case 4: return ring_fwd_launch<T, 4>(P, st);
@@ -922,29 +442,12 @@ template <typename T> static int ring_fwd_typed(const VAParams& P, cudaStream_t 
     default: return ring_fwd_launch<T, 32>(P, st);
   }
 }
-template <typename T> static int ring_bwd_typed(const VAParams& P, int* grid, cudaStream_t st) {
-  switch (ring_lpr<T>(P)) {
-    case 4: return ring_bwd_launch<T, 4>(P, grid, st);
-    case 8: return ring_bwd_launch<T, 8>(P, grid, st);
-    case 16: return ring_bwd_launch<T, 16>(P, grid, st);
-    default: return ring_bwd_launch<T, 32>(P, grid, st);
-  }
-}
-
 int va_ring_fwd(const VAParams& P, int dtype, cudaStream_t st) {
   switch (dtype) {
     case DVA_F32: return ring_fwd_typed<float>(P, st);
     case DVA_BF16: return ring_fwd_typed<__nv_bfloat16>(P, st);
     case DVA_F16: return ring_fwd_typed<__half>(P, st);
     default: return fail(DVA_EINVAL, "view_attention_fwd: unknown dtype");
-  }
-}
-int va_ring_bwd(const VAParams& P, int dtype, int* grid_out, cudaStream_t st) {
-  switch (dtype) {
-    case DVA_F32: return ring_bwd_typed<float>(P, grid_out, st);
-    case DVA_BF16: return ring_bwd_typed<__nv_bfloat16>(P, grid_out, st);
-    case DVA_F16: return ring_bwd_typed<__half>(P, grid_out, st);
-    default: return fail(DVA_EINVAL, "view_attention_bwd: unknown dtype");
   }
 }
 

@@ -102,12 +102,13 @@ int dva_view_attention_fwd(const void* x, const void* idx, int idx_is_i64, const
 
 /* Implementation choice of the fused pair (tuning / test knob, process-wide; results are the same
  * up to fp32 summation order): 0 = auto (default; also DVA_VA_PATH=auto|stream|ring|lane in the
- * environment), 1 = streaming kernels (rows in registers, one point per warp at a time),
- * 2 = ring kernels (rows staged in shared memory by async copies across point boundaries, softmax
- * statistics one lane per point; need G == 4 and rows of whole 16-byte chunks, <= 512 bytes --
- * anything else runs on the streaming kernels whatever the setting), 3 = backward on the
- * lane-per-view kernel (groups of <= 32 views per warp: lane per view for the scores, sub-warp per
- * row for the features; G == 4, rows of 4 / 8 / 16 / 32 chunks), forward as in auto.
+ * environment), 1 = streaming kernels for both passes (rows in registers, one point per warp at a
+ * time), 2 = ring forward (rows staged in shared memory by async copies across point boundaries,
+ * softmax statistics one lane per point; G == 4, rows of whole 16-byte chunks, <= 512 bytes) and
+ * lane-per-view backward (groups of <= 32 views per warp: lane per view for the scores, sub-warp per
+ * row for the features; G == 4, rows of 4 / 8 / 16 / 32 chunks), 3 = streaming forward and
+ * lane-per-view backward.  A pass whose kernel does not apply to the shape runs on the streaming
+ * kernel whatever the setting.
  * TEST / TUNING ONLY: production callers leave it at 0; the choice is a pure function of the shape. */
 int dva_view_attention_set_path(int path);
 
@@ -244,8 +245,7 @@ int dva_linear_gemm(const float* A, const float* B, float* D, int64_t M, int64_t
  *   partials in fp64 (fixed order) into mean / invstd [n_out] (biased variance) and updates the running
  *   buffers (momentum, unbiased variance) like nn.BatchNorm1d.  The apply half is dva_bn_act_fwd with
  *   training = 0 on these mean / invstd.  supported(): 32 <= n_out <= 128, n_out % 4 == 0, k_red >= 8,
- *   k_red % 4 == 0 (the shapes dva_linear_gemm serves with the tcgen05 rows kernel; with DVA_TC_NARROW=0 in the
- *   environment only n_out > 32 and k_red > 32, the round-1 routing); else DVA_EUNSUPPORTED.
+ *   k_red % 4 == 0 (the shapes dva_linear_gemm serves with the tcgen05 rows kernel); else DVA_EUNSUPPORTED.
  * ------------------------------------------------------------------------------------------ */
 int dva_linear_bnstats_supported(int64_t M, int64_t n_out, int64_t k_red);
 size_t dva_linear_bnstats_workspace_bytes(int64_t n_out, int64_t k_red);

@@ -45,7 +45,7 @@ def test_abi_version_and_error_string():
 
 def test_knobs_and_workspace_queries_validate_arguments():
     lib = _lib.load()
-    # implementation choice of the fused pair: 0 auto, 1 streaming, 2 ring, 3 lane (bwd); anything else is refused
+    # kernels of the fused pair: 0 auto, 1 streaming, 2 ring fwd + lane bwd, 3 streaming fwd + lane bwd; anything else is refused
     assert lib.dva_view_attention_set_path(4) == _lib.DVA_EINVAL
     assert lib.dva_view_attention_set_path(-1) == _lib.DVA_EINVAL
     for path in (1, 2, 3, 0):

@@ -24,6 +24,9 @@ CONFIGS = {"config1_s3dis": dict(N=160_000, mean_v=8, C=64), "config3_kitti360":
 
 @pytest.fixture(params=["auto", "stream", "ring", "lane"])
 def path(request):
+    """Kernel pair of the fused view attention (dva_view_attention_set_path): 'auto' = the library's per-shape
+    choice, 'stream' = streaming kernels for both passes, 'ring' = ring forward + lane-per-view backward, 'lane' =
+    streaming forward + lane-per-view backward; 'auto' is restored afterwards."""
     from deepviewagg_b200 import _lib
     lib = _lib.load()
     assert lib.dva_view_attention_set_path({"auto": 0, "stream": 1, "ring": 2, "lane": 3}[request.param]) == 0

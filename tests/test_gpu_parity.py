@@ -97,8 +97,10 @@ def test_segment_edge_cases():
 
 @pytest.fixture(params=["stream", "ring", "lane"])
 def va_path(request):
-    """Run the test once per implementation of the fused pair (streaming kernels / ring kernels /
-    lane-per-view backward, dva_view_attention_set_path); the default 'auto' choice is restored afterwards."""
+    """Run the test once per kernel pair of the fused view attention (dva_view_attention_set_path):
+    'stream' = streaming kernels for both passes, 'ring' = ring forward + lane-per-view backward, 'lane' =
+    streaming forward + lane-per-view backward (ring / lane wherever they apply); the default 'auto' choice
+    is restored afterwards."""
     from deepviewagg_b200 import _lib
     lib = _lib.load()
     assert lib.dva_view_attention_set_path({"stream": 1, "ring": 2, "lane": 3}[request.param]) == 0
@@ -180,7 +182,7 @@ def test_view_attention_long_segments_and_empties(va_path):
     _run_va(64, 3, 128, 4, seed=3, p_empty=0.9)     # mostly unseen points
     _run_va(50, 4, 128, 4, seed=4, p_empty=1.0)     # no view at all (V == 0)
     _run_va(1, 1, 128, 4, seed=8, p_empty=0.0)
-    # ring kernels: segments cut into several pieces at arbitrary batch offsets, 16/32-row batches
+    # ring forward: segments cut into several pieces at arbitrary batch offsets, 16/32-row batches
     _run_va(40, 90, 64, 4, seed=13)
     _run_va(700, 21, 32, 4, seed=14, use_idx=torch.int32)
     _run_va(500, 40, 128, 8, seed=15, dtype=torch.float32)

@@ -54,7 +54,10 @@ def main():
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--groups", type=int, default=4)
     ap.add_argument("--out", default="")
-    ap.add_argument("--path", default="auto", choices=["auto", "stream", "ring", "lane"])
+    ap.add_argument("--path", default="auto", choices=["auto", "stream", "ring", "lane"],
+                    help="kernels of the pair: auto = the library's per-shape choice, stream = streaming kernels for "
+                         "both passes, ring = ring forward + lane backward, lane = streaming forward + lane backward "
+                         "(ring / lane only where they apply)")
     args = ap.parse_args()
     from deepviewagg_b200.host_api import ViewAttentionHostPlan
     from deepviewagg_b200 import _lib
